@@ -2,9 +2,11 @@
 """Throughput benchmark of the detector-simulation hot path (see the task contract in DESIGN.md section "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--events B]
+                    [--dump-outputs DIR]
 
 A *step* is one pass of the whole hot path (`simulate` of detector/simulator.py:52-115 for every event) over one
-batch of B synthetic kinematics events per GPU.  Prints ONE JSON line (rank 0).
+batch of B synthetic kinematics events per GPU.  Prints ONE JSON line (rank 0).  The inputs depend on the arguments
+alone, so `--dump-outputs` of two builds can be compared array for array (see `dump_arrays`).
 
 * value      events/s with the inputs resident in HBM and the results left in HBM (device time, CUDA events
              recorded by the library on its own stream, max over ranks; L2 flushed between steps).
@@ -26,11 +28,14 @@ batch of B synthetic kinematics events per GPU.  Prints ONE JSON line (rank 0).
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import statistics
 import subprocess
 import sys
+import tempfile
 import time
 from pathlib import Path
 
@@ -38,6 +43,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 WORKLOADS = {
     # name: (description, gas, (target, projectile, ejectile), decays [(parent, residual_1)], excitations, beam MeV)
@@ -254,6 +260,31 @@ def reduce_sum(dist, value, device):
     return float(t.item())
 
 
+DUMP_EVENTS = 128  # events whose rows --dump-outputs keeps: ~49 MB at the ~12k points per event of c12aa
+DUMP_BYTES = 64_000_000
+
+
+def dump_arrays(batch, seed=0):
+    """What a caller of the device-resident call gets back (`Engine.read_device_result`: CSR offsets, cloud float64
+    [N, 3], labels int64 [N]), cut to at most DUMP_BYTES as float64 arrays: the point count of every event, and the
+    cloud rows and labels of a fixed, seeded sample of events (`sample_events`, ascending; its tail is dropped should
+    the rows outgrow the budget)."""
+    offsets = batch.offsets
+    counts = np.diff(offsets)
+    sample = np.sort(np.random.default_rng(seed).choice(len(counts), size=min(len(counts), DUMP_EVENTS), replace=False))
+    row_budget = (DUMP_BYTES - 8 * (len(counts) + len(sample)) - 4 * 128) // 32  # 3 cloud columns + label, 8 B each
+    sample = sample[np.cumsum(counts[sample]) <= row_budget]
+    rows = np.concatenate([np.arange(offsets[e], offsets[e + 1]) for e in sample] + [np.zeros(0, np.int64)])
+    return {"points_per_event": counts, "sample_events": sample, "cloud": batch.cloud[rows], "labels": batch.labels[rows]}
+
+
+def write_dump(directory, arrays):
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", np.asarray(a, dtype=np.float64))
+
+
 # ------------------------------------------------------------------------------------------------------- arms
 def run_ours(args):
     import torch
@@ -296,7 +327,7 @@ def run_ours(args):
 
     def step_device(i):
         return eng.simulate_device(mom_dev.data_ptr(), vtx_dev.data_ptr(), B, K, zs, as_, indices, seed=seed + i,
-                                   first_event=first, spyral_rows=args.spyral).stats  # fmt: skip
+                                   first_event=first, spyral_rows=args.spyral)  # fmt: skip
 
     def batch_e2e(i):
         return eng.simulate_batch(mom_pin.numpy(), vtx_pin.numpy(), zs, as_, indices, seed=seed + i, first_event=first,
@@ -346,13 +377,16 @@ def run_ours(args):
     wall0 = time.perf_counter()
     for i in range(args.steps):
         flush_l2()
-        st = step_device(100 + i)
+        last = step_device(100 + i)
+        st = last.stats
         dev_ms += st["ms_total"]
         launches += st["n_kernel_launches"]
         for k, v in st.items():
             stats_sum[k] = stats_sum.get(k, 0) + v
     barrier()
     wall_dev = time.perf_counter() - wall0
+    # the last step's rows stay on the device until the next call on this engine: read back before the e2e legs run
+    dump = dump_arrays(eng.read_device_result(last)) if args.dump_outputs and rank == 0 else None
     # ---- e2e: host buffers in, host buffers out
     barrier()
     e2e_s, e2e_points, e2e_rows, e2e_big = 0.0, 0, 0, 0
@@ -379,7 +413,7 @@ def run_ours(args):
         barrier()
     # ---- e2e in the reference's own return type: float64 [N, 3] + int64 [N] (or float64 [M, 8] Spyral rows) straight
     # from the device, 32 (72 + 8) B/row over PCIe -- what a `SimulationWriter.write` consumer gets without any decode
-    f64_s, f64_steps = None, min(args.steps, 4)
+    f64_s, f64_steps = None, args.steps
     if not args.no_e2e and not args.float64_rows and args.e2e_engines > 1:
         stream_e2e(2, 2000, float64_rows=True, engines=2)  # (sizes the pinned float64 buffers)
         barrier()
@@ -541,6 +575,8 @@ def run_ours(args):
     }  # fmt: skip
     if world == 1 and not args.no_cpu:
         out["cpu_baseline"] = cpu_baseline(args, momenta, vertices)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     print(json.dumps(out), flush=True)
     if dist is not None:
         dist.destroy_process_group()
@@ -557,8 +593,6 @@ def run_pipeline(args):
     first `--writer-chunks` chunks of rank 0 into a scratch directory and reported beside it: a full 10 M-event cloud is
     ~0.9 TB as float64 rows (0.3 TB as typed columns), more than the box can hold or write in minutes.
     """
-    import shutil
-    import tempfile
     import threading
 
     import torch
@@ -829,7 +863,15 @@ def main():
                     help="e2e only: ONE process with a thread and an engine per GPU (0 = off)")
     ap.add_argument("--float64-rows", action="store_true",
                     help="e2e: bring the cloud back as float64[N,3] + int64 labels (32 B/row) instead of typed columns")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed device-resident step computed (rank 0) as DIR/<name>.npy, float64, "
+                         "at most 64 MB: points_per_event, and sample_events / cloud / labels of a seeded event sample")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.thread_gpus > 0 or args.pipeline):
+        ap.error("--dump-outputs applies to the device-resident steps of the default mode")
+    if "NUMBA_CACHE_DIR" not in os.environ:  # numba's on-disk cache (the column decoder) stays out of the tree
+        os.environ["NUMBA_CACHE_DIR"] = tempfile.mkdtemp(prefix="attpc_bench_numba_")
+        atexit.register(shutil.rmtree, os.environ["NUMBA_CACHE_DIR"], ignore_errors=True)
     if args.impl == "reference":
         run_reference(args)
     elif args.thread_gpus > 0:
