@@ -12,7 +12,7 @@ from pathlib import Path
 
 LIB_NAME = "libattpc_b200.so"
 LIB_PATH = Path(__file__).resolve().parent / LIB_NAME
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 # flags (include/attpc_b200.h)
 KEEP_ALL_TB = 1 << 0
@@ -54,6 +54,7 @@ class AttpcConfig(C.Structure):
         ("copy_events_per_launch", C.c_int32),
         ("unit_points", C.c_int32),
         ("table_spill_keys", C.c_int32),
+        ("longitudinal_diffusion", C.c_double),
     ]
 
 

@@ -77,6 +77,9 @@ struct PinnedArray {
 }  // namespace
 
 constexpr int64_t ATTPC_BIG_CAP = 1 << 20;  // (row, count) exceptions of the compact electrons column per call
+// Groups per chunk when points are split into sub-points: bounds the sub-point records (160 B each, up to
+// long_buckets per point) held at once, at the price of more (shorter) launches
+constexpr int64_t SUB_CHUNK_GROUPS = 4;
 
 struct AttpcSim {
     int device = 0;
@@ -137,6 +140,13 @@ struct AttpcSim {
     DevArray<unsigned> pstart, n_entries, mode;
     int32_t ranks = 1;
     int32_t max_units = 0;
+    // longitudinal diffusion (P.long_diffusion > 0): geom / rec then hold the SUB-POINTS (one per time bucket of a
+    // point's window) of one chunk of at most SUB_CHUNK_GROUPS groups, sub_cap per group
+    int64_t sub_cap = 0;
+    int32_t long_buckets = 0;   // most buckets one point can spread over: floor(6 sigma_L) + 2 at windows_edge + 1
+    int32_t sub_max_units = 0;  // work units per group over sub-points
+    DevArray<unsigned> nsub, sub_cnt, sub_start;  // per point: sub-point offset in its list; per (event, rank) list
+    DevArray<unsigned long long> sub_total;       // [SUB_CHUNK_GROUPS] sub-points per group of the chunk
     DevArray<HashEntry> hash;
     DevArray<uint64_t> sort_items;
     DevArray<uint4> staged;  // ordered rows of the chunk's events between order_kernel and emit_kernel
@@ -252,19 +262,35 @@ int ensure_work_buffers(AttpcSim* sim, int64_t launch_events, int32_t ranks, int
         CU(ls.counters.reserve(1));
         CU(ls.counters_host.reserve(1));
     }
-    CU(sim->geom.reserve(pts * GEOM_DOUBLES));
-    CU(sim->rec.reserve(pts * REC_WORDS));
     sim->max_units = (int32_t)(sim->group_events + sim->group_point_cap / sim->unit_points + 1);
-    CU(sim->unit_event.reserve(n_groups * sim->max_units));
-    CU(sim->unit_first.reserve(n_groups * sim->max_units));
-    CU(sim->unit_count.reserve(n_groups * sim->max_units));
-    CU(sim->unit_order.reserve(n_groups * sim->max_units));
+    int64_t units = sim->max_units;
+    if (sim->P.long_diffusion > 0.0) {
+        // first guess 256 points per event, each spread over long_buckets; grown on overflow (overflow_sub)
+        if (sim->sub_cap == 0) sim->sub_cap = (int64_t)sim->group_events * 256 * std::min(sim->long_buckets, 16);
+        const int64_t subs = std::min<int64_t>(n_groups, SUB_CHUNK_GROUPS) * sim->sub_cap;
+        CU(sim->geom.reserve(subs * GEOM_DOUBLES));
+        CU(sim->rec.reserve(subs * REC_WORDS));
+        CU(sim->nsub.reserve(pts));
+        CU(sim->sub_cnt.reserve(launch_events * ranks));
+        CU(sim->sub_start.reserve(launch_events * ranks));
+        CU(sim->sub_total.reserve(SUB_CHUNK_GROUPS));
+        sim->sub_max_units = (int32_t)(sim->group_events + sim->sub_cap / sim->unit_points + 1);
+        units = std::max<int64_t>(units, sim->sub_max_units);
+    } else {
+        CU(sim->geom.reserve(pts * GEOM_DOUBLES));
+        CU(sim->rec.reserve(pts * REC_WORDS));
+    }
+    CU(sim->unit_event.reserve(n_groups * units));
+    CU(sim->unit_first.reserve(n_groups * units));
+    CU(sim->unit_count.reserve(n_groups * units));
+    CU(sim->unit_order.reserve(n_groups * units));
     CU(sim->n_units.reserve(n_groups));
     CU(sim->pstart.reserve(launch_events * ranks));
     CU(sim->n_entries.reserve(launch_events));
     CU(sim->mode.reserve(launch_events));
     // tables and sort scratch for one chunk of groups (run_groups)
-    const int64_t table_groups = std::min<int64_t>(n_groups, std::max<int64_t>(1, chunk_groups));
+    int64_t table_groups = std::min<int64_t>(n_groups, std::max<int64_t>(1, chunk_groups));
+    if (sim->P.long_diffusion > 0.0) table_groups = std::min<int64_t>(table_groups, SUB_CHUNK_GROUPS);  // run_groups' chunks
     CU(sim->hash.reserve(table_groups * sim->group_events * sim->hash_cap));
     CU(sim->sort_items.reserve(table_groups * sim->group_events * scratch_stride(sim->hash_cap)));
     CU(sim->staged.reserve(table_groups * sim->group_events * sim->hash_cap));
@@ -321,6 +347,22 @@ PointBuf point_buf(AttpcSim* sim, int which) {
     pb.group_events = sim->group_events;
     pb.ranks = sim->ranks;
     return pb;
+}
+
+// The sub-points of the chunk whose first group is g0 (longitudinal diffusion), as the point_scan and deposit kernels
+// read points: records from sim->rec / sim->geom, lists counted in sub_cnt, groups numbered from 0 inside the chunk.
+PointBuf sub_buf(AttpcSim* sim, int which, int64_t g0) {
+    PointBuf sb = point_buf(sim, which);
+    sb.cnt = sim->sub_cnt.p;
+    sb.start = sim->sub_start.p;
+    sb.max_units = sim->sub_max_units;
+    sb.unit_event += g0 * sb.max_units;
+    sb.unit_first += g0 * sb.max_units;
+    sb.unit_count += g0 * sb.max_units;
+    sb.unit_order += g0 * sb.max_units;
+    sb.n_units += g0;
+    sb.group_cap = sim->sub_cap;
+    return sb;
 }
 
 template <bool RECORD>
@@ -394,7 +436,9 @@ int run_groups(AttpcSim* sim, int64_t launch_events, FinalizeArgs fa, int which,
     // Groups are processed in chunks: every kernel is launched once per chunk with one grid row per group, so the
     // ramp-up and tail of a launch are paid once per chunk.  When rows go to the host a chunk is what is copied while
     // the next chunk computes; otherwise it is as many groups as the tables are sized for.
-    const int64_t gpc = std::max<int64_t>(1, fences ? groups_per_chunk : sim->chunk_groups);
+    const bool split = sim->P.long_diffusion > 0.0;
+    int64_t gpc = std::max<int64_t>(1, fences ? groups_per_chunk : sim->chunk_groups);
+    if (split) gpc = std::min<int64_t>(gpc, SUB_CHUNK_GROUPS);
     for (int64_t g0 = 0; g0 < n_groups; g0 += gpc) {
         const int64_t ng = std::min<int64_t>(gpc, n_groups - g0);
         GroupView gv;
@@ -410,13 +454,32 @@ int run_groups(AttpcSim* sim, int64_t launch_events, FinalizeArgs fa, int which,
         gv.chunk_e0 = 0;
         gv.spill_keys = sim->spill_keys;
         cudaEvent_t d0 = sim->mark();
+        const dim3 point_grid((unsigned)std::max<int64_t>(1, sim->sm_count * 4 / ng), (unsigned)ng);
         point_scan_kernel<<<(unsigned)ng, 1024, 0, sim->stream>>>(pb, gv, ctr);
-        point_order_kernel<<<dim3((unsigned)std::max<int64_t>(1, sim->sm_count * 4 / ng), (unsigned)ng), 256, 0,
-                             sim->stream>>>(sim->P, pb, gv, ctr);
+        if (!split) {
+            point_order_kernel<<<point_grid, 256, 0, sim->stream>>>(sim->P, pb, gv, ctr);
+        } else {  // points -> one sub-point per time bucket of their window, then units over sub-points
+            PointBuf sb = sub_buf(sim, which, g0);
+            GroupView gvs = gv;
+            gvs.group = 0;
+            CU(cudaMemsetAsync(sim->sub_total.p, 0, (size_t)ng * sizeof(unsigned long long), sim->stream));
+            sub_count_kernel<<<point_grid, 256, 0, sim->stream>>>(sim->P, pb, gv, ctr, sim->nsub.p);
+            sub_scan_kernel<<<point_grid, 256, 0, sim->stream>>>(pb, sb, gv, ctr, sim->nsub.p, sim->sub_total.p);
+            point_scan_kernel<<<(unsigned)ng, 1024, 0, sim->stream>>>(sb, gvs, ctr);
+            sub_point_kernel<<<point_grid, 256, 0, sim->stream>>>(sim->P, pb, sb, gv, ctr, sim->nsub.p);
+            sim->launches += 3;
+        }
         CU(cudaMemsetAsync(sim->n_entries.p + gv.first_slot, 0, (size_t)gv.n_events * sizeof(unsigned), sim->stream));
         cudaEvent_t k0 = sim->mark();
-        deposit_kernel<<<dim3((unsigned)sim->max_units, (unsigned)ng), DEPOSIT_THREADS, DEPOSIT_SMEM_BYTES,
-                         sim->stream>>>(sim->P, pb, gv, ctr);
+        if (!split) {
+            deposit_kernel<<<dim3((unsigned)sim->max_units, (unsigned)ng), DEPOSIT_THREADS, DEPOSIT_SMEM_BYTES,
+                             sim->stream>>>(sim->P, pb, gv, ctr);
+        } else {
+            GroupView gvs = gv;
+            gvs.group = 0;
+            deposit_kernel<<<dim3((unsigned)sim->sub_max_units, (unsigned)ng), DEPOSIT_THREADS, DEPOSIT_SMEM_BYTES,
+                             sim->stream>>>(sim->P, sub_buf(sim, which, g0), gvs, ctr);
+        }
         cudaEvent_t d1 = sim->mark();
         CU(cudaMemsetAsync(qbase, 0, 4 * sizeof(unsigned), sim->stream));
         order_kernel<<<(unsigned)gv.n_events, FIN_THREADS, FIN_SMEM_BYTES, sim->stream>>>(sim->P, fa, gv, ctr);
@@ -901,7 +964,13 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
             if (++retries > 24) return sim->fail(ATTPC_E_CAPACITY, "buffers still too small after 24 retries");
             CU(cudaStreamSynchronize(T));  // the next launch's track kernel may be using buffers we are about to free
             CU(cudaStreamSynchronize(C));
-            if (now.overflow_points) {
+            if (now.overflow_sub) {  // (overflow_points is raised with it: the point lists themselves were complete)
+                if (sim->sub_cap >= (1LL << 30)) return sim->fail(ATTPC_E_CAPACITY, "a group needs > 2^30 sub-points");
+                sim->sub_cap *= 2;
+                sim->geom.release(); sim->rec.release();
+                sim->unit_event.release(); sim->unit_first.release(); sim->unit_count.release();
+                sim->unit_order.release();
+            } else if (now.overflow_points) {
                 sim->group_point_cap *= 2;
                 for (auto& s2 : sim->slot) s2.release_points();
                 sim->geom.release(); sim->rec.release();
@@ -1122,6 +1191,7 @@ void attpc_destroy(AttpcSim* sim) {
     sim->resp_sorted.release(); sim->resp_prefix.release(); sim->tables.release(); sim->stop_ns.release(); sim->plan_cls.release(); sim->plan_counts.release(); sim->plan_order.release();
     sim->hash.release(); sim->sort_items.release(); sim->staged.release(); sim->big_list.release();
     sim->geom.release(); sim->rec.release();
+    sim->nsub.release(); sim->sub_cnt.release(); sim->sub_start.release(); sim->sub_total.release();
     sim->unit_event.release(); sim->unit_first.release(); sim->unit_count.release(); sim->unit_order.release();
     sim->n_units.release();
     sim->pstart.release(); sim->n_entries.release(); sim->mode.release();
@@ -1162,6 +1232,10 @@ int attpc_create(const AttpcConfig* cfg, const int16_t* pad_lut, const double* p
         g_create_error = "attpc_create: windows_edge == micromegas_edge, drift_velocity <= 0 or w_value <= 0";
         return ATTPC_E_BADARG;
     }
+    if (!(cfg->longitudinal_diffusion >= 0.0) || !std::isfinite(cfg->longitudinal_diffusion)) {
+        g_create_error = "attpc_create: longitudinal_diffusion must be finite and >= 0";
+        return ATTPC_E_BADARG;
+    }
     cudaError_t e = cudaSetDevice(device);
     if (e != cudaSuccess) {
         g_create_error = std::string("cudaSetDevice: ") + cudaGetErrorString(e);
@@ -1196,6 +1270,16 @@ int attpc_create(const AttpcConfig* cfg, const int16_t* pad_lut, const double* p
     P.mm_edge = (double)cfg->micromegas_edge;
     P.win_edge = (double)cfg->windows_edge;
     P.diffusion = cfg->diffusion;
+    P.long_diffusion = cfg->longitudinal_diffusion;
+    if (P.long_diffusion > 0.0) {  // widest window: sigma_L one bucket past the window edge (no point drifts longer)
+        const double t = P.win_edge + 1.0;
+        const double sl = std::sqrt(2.0 * P.long_diffusion * P.dv * t / cfg->efield) / P.dv;
+        if (!(sl < 1.0e6)) {
+            sim->fail(ATTPC_E_BADARG, "attpc_create: longitudinal diffusion needs efield > 0 (sigma_L = %g)", sl);
+            return bail(ATTPC_E_BADARG);
+        }
+        sim->long_buckets = (int32_t)std::floor(6.0 * sl) + 2;
+    }
     P.efield = cfg->efield;
     P.fano = cfg->fano_factor;
     P.ev_per_w = 1.0e6 / cfg->w_value;

@@ -9,6 +9,8 @@
 //                     reference's exact operation order (parity part (a)).
 //   point_scan/order  per-event work units, points into (event, rank, arrival) order, sigma_t and the pad-table rows and
 //                     columns of the 10x10 mesh of every point (detector/transporter.py:78-120, 217-226, 301).
+//   sub_*             longitudinal diffusion only (off by default, not in the reference): every point becomes one
+//                     record per time bucket of its window ("sub-points"), which the deposit kernel takes as points.
 //   deposit_kernel    one CTA per work unit, one lane per mesh row: pad lookup, bivariate-normal share, accumulation
 //                     per (pad, time bucket) in a shared-memory open-addressing table that is appended to the event's
 //                     entry list in dense segments (detector/transporter.py:11-41, 123-249, 252-317; pairing.py:6-28).
@@ -80,6 +82,7 @@ struct SimParams {
     double mesh_w[MESH_N * MESH_N];  // (2 / (9 pi)) exp(-(a_i^2 + a_j^2) / 2), a_i = -3 + 6 i / 9: pdf * step^2 of the mesh
     double mesh_w_unique[MESH_N * MESH_N];  // its distinct values (15 for the symmetric 10 x 10 mesh)
     int32_t n_mesh_w_unique, pad1;
+    double long_diffusion;  // V, longitudinal diffusion coefficient (0: off, every point stays in one time bucket)
 };
 
 // Active track points (>= 1 electron).  The track kernels append them per event group in arrival order and number
@@ -115,7 +118,9 @@ struct PointBuf {
 struct Counters {
     unsigned long long track_cursor;
     unsigned long long traj_points, active_points, primary_electrons, deposits, keys, probes, flushes;
-    int overflow_points, overflow_hash, overflow_out, replay_miss, overflow_charge, pad_;
+    // overflow_sub: the sub-points of longitudinal diffusion did not fit (raised together with overflow_points, which
+    // voids the launch; the host then grows the sub-point buffers instead of the point buffers)
+    int overflow_points, overflow_hash, overflow_out, replay_miss, overflow_charge, overflow_sub;
     // integrator probes: Dormand-Prince steps tried / rejected, and the most loop passes any one track needed (the
     // serial critical path of a launch)
     unsigned long long rk_steps, rk_rejects, max_track_passes;
@@ -1127,7 +1132,9 @@ __device__ __forceinline__ int lut_index(const SimParams& P, double coord_m) {
 //   word 14     rank of the track (position in `indices`)
 constexpr int REC_WORDS = 16;
 
-__device__ __forceinline__ void make_point(const SimParams& P, double cx, double cy, double time, long long q,
+// `tb` is the time bucket of the record: (int)time (detector/transporter.py:165, 238), or one bucket of the
+// longitudinal window of the point (sub_point_kernel); `q` its electrons.
+__device__ __forceinline__ void make_point(const SimParams& P, double cx, double cy, double time, int tb, long long q,
                                            bool exact_mesh, double* g, uint32_t* rec) {
     g[0] = cx;
     g[1] = cy;
@@ -1138,7 +1145,6 @@ __device__ __forceinline__ void make_point(const SimParams& P, double cx, double
     rec[3] = (uint32_t)__double2hiint(g[10]);
     // detector/transporter.py:301, evaluated left to right
     const double sigma = __dsqrt_rn(__ddiv_rn(__dmul_rn(__dmul_rn(__dmul_rn(2.0, P.diffusion), P.dv), time), P.efield));
-    const int tb = (int)time;  // detector/transporter.py:165, 238
     if (tb < 0 || tb >= 8192 || !(sigma == sigma)) return;  // kind 0: never reached for 0 <= z <= length + mm_edge*dv (tb <= windows_edge)
     if (sigma == 0.0) {  // kind 1: single deposit, transporter.py:123-169
         rec[0] = (uint32_t)tb | (1u << 30);
@@ -1209,7 +1215,7 @@ __global__ void __launch_bounds__(256) point_order_kernel(const __grid_constant_
         uint32_t rec[REC_WORDS];
 #pragma unroll
         for (int k = 0; k < GEOM_DOUBLES; ++k) g[k] = 0.0;
-        make_point(P, pb.x[i], pb.y[i], pb.t[i], pb.q[i], gv.exact_mesh != 0, g, rec);
+        make_point(P, pb.x[i], pb.y[i], pb.t[i], (int)pb.t[i], pb.q[i], gv.exact_mesh != 0, g, rec);
         rec[14] = (uint32_t)pb.rank[i];
         if ((rec[0] >> 29) & 1u) {  // only the exact path of the deposit kernel reads the mesh constants
             double2* out = reinterpret_cast<double2*>(pb.geom + d * GEOM_DOUBLES);
@@ -1219,6 +1225,134 @@ __global__ void __launch_bounds__(256) point_order_kernel(const __grid_constant_
         uint4* out_rec = reinterpret_cast<uint4*>(pb.rec + d * REC_WORDS);
 #pragma unroll
         for (int k = 0; k < REC_WORDS / 4; ++k) out_rec[k] = make_uint4(rec[4 * k], rec[4 * k + 1], rec[4 * k + 2], rec[4 * k + 3]);
+    }
+}
+
+// ------------------------------------------------------------------------------------- longitudinal diffusion
+// (an extension outside the reference, DESIGN.md §3a; launched only when SimParams.long_diffusion > 0)
+// A point of drift time `time` [time buckets] spreads over the buckets k0..k1 = floor(time -+ 3 sigma_L) (k < 0
+// dropped) with sigma_L = sqrt(2 D_L dv time / E) / dv, the transverse expression of detector/transporter.py:301 over
+// dv.  Bucket k receives (int64)(f_k q), f_k = Phi((k + 1 - time) / sigma_L) - Phi((k - time) / sigma_L), and every
+// bucket of the window becomes a record of its own ("sub-point") with the point's position and transverse sigma, so
+// the deposit kernel runs unchanged on one time bucket and at most 100 keys per record.  The window depends on the
+// correctly rounded sqrt and floor only; erfc decides the charges, not which keys exist.
+// sigma_L <= 0 or NaN (time <= 0): the point keeps its single bucket (int)time and all its electrons.
+__device__ __forceinline__ double long_sigma(const SimParams& P, double time) {
+    return __ddiv_rn(__dsqrt_rn(__ddiv_rn(__dmul_rn(__dmul_rn(__dmul_rn(2.0, P.long_diffusion), P.dv), time), P.efield)),
+                     P.dv);
+}
+
+__device__ __forceinline__ void long_window(const SimParams& P, double time, double& sl, int& k0, int& k1) {
+    sl = long_sigma(P, time);
+    if (!(sl > 0.0)) {
+        k0 = k1 = (int)time;
+        return;
+    }
+    const double w = __dmul_rn(3.0, sl);
+    k0 = max(0, (int)floor(__dsub_rn(time, w)));
+    k1 = (int)floor(__dadd_rn(time, w));
+}
+
+__device__ __forceinline__ double long_phi(double x) {  // 0.5 erfc(-x / sqrt(2))
+    return __dmul_rn(0.5, erfc(__ddiv_rn(-x, 1.4142135623730951)));
+}
+
+__device__ __forceinline__ long long long_electrons(double time, double sl, int k, long long q) {
+    const double f = __dsub_rn(long_phi(__ddiv_rn(__dsub_rn((double)(k + 1), time), sl)),
+                               long_phi(__ddiv_rn(__dsub_rn((double)k, time), sl)));
+    return (long long)__dmul_rn(f, (double)q);
+}
+
+// (1) sub-points of every point, stored at the point's position in the (event, rank, arrival) order
+__global__ void __launch_bounds__(256) sub_count_kernel(const __grid_constant__ SimParams P, PointBuf pb,
+                                                        GroupView chunk, const Counters* ctr, unsigned* nsub) {
+    if (ctr->overflow_points) return;
+    const GroupView gv = sub_group(chunk, blockIdx.y);
+    const int64_t n = min((int64_t)pb.count[gv.group], pb.group_cap);
+    const int64_t base = (int64_t)gv.group * pb.group_cap;
+    for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t i = base + p;
+        double sl;
+        int k0, k1;
+        long_window(P, pb.t[i], sl, k0, k1);
+        nsub[base + pb.start[(int64_t)pb.ev[i] * pb.ranks + pb.rank[i]] + pb.j[i]] = k1 >= k0 ? (unsigned)(k1 - k0 + 1) : 0u;
+    }
+}
+
+// (2) one warp per (event, rank) list: exclusive scan of the list's sub-point counts in place (the offset of each
+// point's first sub-point inside the list) and the list's total in sb.cnt, which point_scan_kernel then turns into
+// sub-point list starts and work units.  The group's total is checked against the sub-point capacity sb.group_cap.
+__global__ void __launch_bounds__(256) sub_scan_kernel(PointBuf pb, PointBuf sb, GroupView chunk, Counters* ctr,
+                                                       unsigned* nsub, unsigned long long* sub_total) {
+    if (ctr->overflow_points) return;
+    const GroupView gv = sub_group(chunk, blockIdx.y);
+    const int lane = threadIdx.x & 31;
+    const int n = gv.n_events * pb.ranks;
+    const int64_t first = (int64_t)gv.first_slot * pb.ranks;
+    const int64_t base = (int64_t)gv.group * pb.group_cap;
+    const int n_warps = gridDim.x * (blockDim.x / 32);
+    for (int l = blockIdx.x * (blockDim.x / 32) + (threadIdx.x >> 5); l < n; l += n_warps) {
+        const int64_t s = base + pb.start[first + l];
+        const unsigned c = pb.cnt[first + l];
+        unsigned run = 0;
+        for (unsigned o = 0; o < c; o += 32) {
+            const unsigned idx = o + (unsigned)lane;
+            const unsigned v = idx < c ? nsub[s + idx] : 0u;
+            unsigned x = v;
+#pragma unroll
+            for (int k = 1; k < 32; k <<= 1) {
+                const unsigned y = __shfl_up_sync(FULL, x, k);
+                if (lane >= k) x += y;
+            }
+            if (idx < c) nsub[s + idx] = run + x - v;
+            run += __shfl_sync(FULL, x, 31);
+        }
+        if (lane == 0) {
+            sb.cnt[first + l] = run;
+            const unsigned long long before = run ? atomicAdd(&sub_total[blockIdx.y], (unsigned long long)run) : 0ull;
+            if (before + run > (unsigned long long)sb.group_cap) {  // the host grows the sub-point buffers and redoes the launch
+                ctr->overflow_sub = 1;
+                ctr->overflow_points = 1;
+            }
+        }
+    }
+}
+
+// (3) after point_scan_kernel on sb: the records of every sub-point, (event, rank, arrival, bucket) order.  `sb`
+// addresses the chunk's groups from 0 (its records exist for one chunk at a time).
+__global__ void __launch_bounds__(256) sub_point_kernel(const __grid_constant__ SimParams P, PointBuf pb, PointBuf sb,
+                                                        GroupView chunk, const Counters* ctr, const unsigned* nsub) {
+    if (ctr->overflow_points) return;
+    const GroupView gv = sub_group(chunk, blockIdx.y);
+    const int64_t n = min((int64_t)pb.count[gv.group], pb.group_cap);
+    const int64_t base = (int64_t)gv.group * pb.group_cap;
+    const int64_t sbase = (int64_t)blockIdx.y * sb.group_cap;
+    for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (int64_t)gridDim.x * blockDim.x) {
+        const int64_t i = base + p;
+        const int64_t l = (int64_t)pb.ev[i] * pb.ranks + pb.rank[i];
+        const double time = pb.t[i], cx = pb.x[i], cy = pb.y[i];
+        const long long q = pb.q[i];
+        double sl;
+        int k0, k1;
+        long_window(P, time, sl, k0, k1);
+        int64_t d = sbase + sb.start[l] + nsub[base + pb.start[l] + pb.j[i]];
+        for (int k = k0; k <= k1; ++k, ++d) {
+            double g[GEOM_DOUBLES];
+            uint32_t rec[REC_WORDS];
+#pragma unroll
+            for (int m = 0; m < GEOM_DOUBLES; ++m) g[m] = 0.0;
+            make_point(P, cx, cy, time, k, sl > 0.0 ? long_electrons(time, sl, k, q) : q, gv.exact_mesh != 0, g, rec);
+            rec[14] = (uint32_t)pb.rank[i];
+            if ((rec[0] >> 29) & 1u) {
+                double2* out = reinterpret_cast<double2*>(sb.geom + d * GEOM_DOUBLES);
+#pragma unroll
+                for (int m = 0; m < GEOM_DOUBLES / 2; ++m) out[m] = make_double2(g[2 * m], g[2 * m + 1]);
+            }
+            uint4* out_rec = reinterpret_cast<uint4*>(sb.rec + d * REC_WORDS);
+#pragma unroll
+            for (int m = 0; m < REC_WORDS / 4; ++m)
+                out_rec[m] = make_uint4(rec[4 * m], rec[4 * m + 1], rec[4 * m + 2], rec[4 * m + 3]);
+        }
     }
 }
 

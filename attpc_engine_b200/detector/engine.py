@@ -256,6 +256,9 @@ class Engine:
             raise ValueError("Pad grid is not loaded")  # solver.py:400-401
         if config.pad_centers is None or config.pad_sizes is None:
             raise ValueError("Pad centers are not assigned")  # writer.py:220-221
+        long_diffusion = float(getattr(config.det_params, "longitudinal_diffusion", 0.0))
+        if not (math.isfinite(long_diffusion) and long_diffusion >= 0.0):
+            raise ValueError(f"longitudinal_diffusion must be finite and >= 0, got {long_diffusion}")
         self.lib = _lib.load()
         self.config = config
         self.device = int(device)
@@ -279,6 +282,7 @@ class Engine:
         cfg.bfield = float(det.bfield)
         cfg.mpgd_gain = int(det.mpgd_gain)
         cfg.diffusion = float(det.diffusion)
+        cfg.longitudinal_diffusion = long_diffusion
         cfg.fano_factor = float(det.fano_factor)
         cfg.w_value = float(det.w_value)
         cfg.gas_density = float(target.density)
@@ -334,6 +338,7 @@ class Engine:
         cfg.length = float(length)
         cfg.efield, cfg.bfield, cfg.mpgd_gain = 1.0, 0.0, 1
         cfg.diffusion, cfg.fano_factor, cfg.w_value, cfg.gas_density = 0.0, 0.0, 1.0, 0.0
+        cfg.longitudinal_diffusion = 0.0
         cfg.micromegas_edge, cfg.windows_edge = int(mm_edge), int(window_edge)
         cfg.adc_threshold = float(threshold)
         cfg.drift_velocity = float(length) / float(int(window_edge) - int(mm_edge))
@@ -711,7 +716,7 @@ def config_fingerprint(config: Config, nuclei: list) -> tuple:
         float(det.length), float(det.efield), float(det.bfield), int(det.mpgd_gain), float(det.diffusion),
         float(det.fano_factor), float(det.w_value), float(elec.clock_freq), float(elec.amp_gain),
         float(elec.shaping_time), int(elec.micromegas_edge), int(elec.windows_edge), float(elec.adc_threshold),
-        float(config.drift_velocity),
+        float(config.drift_velocity), float(getattr(det, "longitudinal_diffusion", 0.0)),
     )  # fmt: skip
     target = det.gas_target
     probes = tuple(

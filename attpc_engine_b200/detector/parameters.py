@@ -33,7 +33,13 @@ class DetectorParams:
     """Detector parameters (`parameters.py:10-48`).
 
     length [m], efield [V/m], bfield [T], mpgd_gain (int, unitless), gas_target,
-    diffusion [V] (transverse), fano_factor, w_value [eV].
+    diffusion [V] (transverse), fano_factor, w_value [eV], longitudinal_diffusion [V].
+
+    ``longitudinal_diffusion`` is an extension (the reference has no such field) and the last
+    field, so that the reference's eight positional arguments still work.  It spreads every
+    ionisation point over the time buckets ``floor(t -+ 3 sigma_L)``, with
+    ``sigma_L = sqrt(2 D_L dv t / efield) / dv`` time buckets after a drift of ``t`` buckets; the
+    default 0 keeps the reference's one bucket per point (see DESIGN.md §3a).
     """
 
     length: float
@@ -44,6 +50,7 @@ class DetectorParams:
     diffusion: float
     fano_factor: float
     w_value: float
+    longitudinal_diffusion: float = 0.0
 
 
 @dataclass

@@ -20,7 +20,7 @@
 extern "C" {
 #endif
 
-#define ATTPC_ABI_VERSION 7
+#define ATTPC_ABI_VERSION 8
 
 enum {
     ATTPC_OK = 0,
@@ -90,6 +90,12 @@ typedef struct AttpcConfig {
     /* stress knobs for tests (0 = library default; values above the default are clamped): results never depend on them */
     int32_t unit_points;            /* points of one event handled by one CTA of the deposit kernel (default 1024) */
     int32_t table_spill_keys;       /* keys in a CTA's shared-memory table that trigger an append to the event's list */
+    /* longitudinal diffusion (an extension: the reference has none), V, same meaning as `diffusion`; 0 = off, the
+       reference's behaviour.  A point of drift time t [time buckets] is spread over the buckets
+       floor(t -+ 3 sigma_L), sigma_L = sqrt(2 D_L dv t / efield) / dv, bucket k receiving
+       (int64)(q (Phi((k + 1 - t) / sigma_L) - Phi((k - t) / sigma_L))) electrons; every bucket of the window
+       then goes through the transverse 10x10 mesh like a point of its own ("sub-point").  Must be finite, >= 0. */
+    double longitudinal_diffusion;
 } AttpcConfig;
 
 /* One ion species: the dE/dx table of attpc_engine_b200/target.py:DedxTable (pseudo-log grid). */
@@ -133,7 +139,8 @@ typedef struct AttpcResult {
     int64_t n_trajectory_points; /* 0.1 ns grid points emitted by the integrator */
     int64_t n_active_points;     /* points with >= 1 electron (detector/solver.py:387) */
     int64_t n_primary_electrons; /* sum of those electrons before mpgd_gain */
-    int64_t n_deposits;          /* pixel deposits attempted (100 per active point when sigma > 0) */
+    int64_t n_deposits;          /* pixel deposits attempted (100 per active point when sigma > 0; with longitudinal
+                                    diffusion 100 per sub-point, i.e. per time bucket of each point's window) */
     int64_t n_keys;              /* distinct (pad, tb) keys before the time-bucket mask */
     /* device time of each stage in ms (CUDA events on the library's stream) */
     float ms_h2d, ms_tracks, ms_deposit, ms_finalize, ms_d2h, ms_total;
@@ -160,7 +167,8 @@ typedef struct AttpcResult {
     int64_t n_big;                   /* rows whose count is >= 2^32 */
     const int64_t* big_rows;         /* [n_big] row index (unordered) */
     const int64_t* big_electrons;    /* [n_big] full count of that row */
-    float ms_order;              /* device time of the point ordering kernels (scan + scatter) before the deposit kernel;
+    float ms_order;              /* device time of the point ordering kernels (scan + scatter, and with longitudinal
+                                    diffusion the split into sub-points) before the deposit kernel;
                                     ms_deposit is the deposit kernel alone */
     float reserved2;
     /* ATTPC_SPYRAL_COLUMNS: rows [row_offsets[e], row_offsets[e+1]) of event e, in the order of `rows` */
