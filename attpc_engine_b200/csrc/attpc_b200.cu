@@ -11,6 +11,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/attpc_b200.h"
@@ -30,6 +31,19 @@ template <typename T>
 struct DevArray {
     T* p = nullptr;
     int64_t n = 0;
+    DevArray() = default;
+    DevArray(const DevArray&) = delete;
+    DevArray& operator=(const DevArray&) = delete;
+    DevArray(DevArray&& o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
+    DevArray& operator=(DevArray&& o) noexcept {
+        if (this != &o) {
+            release();
+            p = std::exchange(o.p, nullptr);
+            n = std::exchange(o.n, 0);
+        }
+        return *this;
+    }
+    ~DevArray() { release(); }
     cudaError_t reserve(int64_t want, bool keep = false, cudaStream_t s = 0) {
         if (want <= n) return cudaSuccess;
         T* q = nullptr;
@@ -55,6 +69,19 @@ template <typename T>
 struct PinnedArray {
     T* p = nullptr;
     int64_t n = 0;
+    PinnedArray() = default;
+    PinnedArray(const PinnedArray&) = delete;
+    PinnedArray& operator=(const PinnedArray&) = delete;
+    PinnedArray(PinnedArray&& o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
+    PinnedArray& operator=(PinnedArray&& o) noexcept {
+        if (this != &o) {
+            release();
+            p = std::exchange(o.p, nullptr);
+            n = std::exchange(o.n, 0);
+        }
+        return *this;
+    }
+    ~PinnedArray() { release(); }
     cudaError_t reserve(int64_t want, bool keep = false) {
         if (want <= n) return cudaSuccess;
         want += want / 4;  // pinning is slow (~0.5 s/GB): grow with slack so that it is rare
@@ -72,6 +99,28 @@ struct PinnedArray {
         p = nullptr;
         n = 0;
     }
+};
+
+// An output with one row per cloud row or per Spyral row: the device array the kernels write, the pinned mirror its
+// rows are copied to, and the bytes of one row.  Sink<T, W> (W values of type T per row) gives typed access.
+struct RowSink {
+    DevArray<char> dev;
+    PinnedArray<char> host;
+    const int64_t row_bytes;
+    explicit RowSink(int64_t bytes) : row_bytes(bytes) {}
+    cudaError_t reserve(int64_t rows, bool keep, cudaStream_t s) { return dev.reserve(rows * row_bytes, keep, s); }
+    cudaError_t reserve_host(int64_t rows, bool keep) { return host.reserve(rows * row_bytes, keep); }
+    cudaError_t copy_to_host(int64_t first, int64_t rows, cudaStream_t s) {
+        return cudaMemcpyAsync(host.p + first * row_bytes, dev.p + first * row_bytes, (size_t)(rows * row_bytes),
+                               cudaMemcpyDeviceToHost, s);
+    }
+};
+
+template <typename T, int W = 1>
+struct Sink : RowSink {
+    Sink() : RowSink(W * (int64_t)sizeof(T)) {}
+    T* d() const { return reinterpret_cast<T*>(dev.p); }
+    T* h() const { return reinterpret_cast<T*>(host.p); }
 };
 
 }  // namespace
@@ -123,10 +172,6 @@ struct AttpcSim {
         void release_points() {
             px.release(); py.release(); pt.release(); pq.release(); pev.release(); prank.release(); pj.release();
         }
-        void release_all() {
-            release_points();
-            group_count.release(); pcnt.release(); counters.release(); counters_host.release();
-        }
     } slot[2];
     cudaStream_t stream_t = nullptr, stream_c = nullptr;  // track kernels, device-to-host copies
     std::vector<cudaEvent_t> sync_events;                 // untimed events for cross-stream ordering
@@ -155,41 +200,43 @@ struct AttpcSim {
     DevArray<unsigned> kept;
     DevArray<double> in_momenta, in_vertices;
 
-    // outputs
-    DevArray<int16_t> col_pad_dev;
-    DevArray<uint32_t> col_tbq_dev;
-    DevArray<int64_t> col_q_dev, big_rows_dev, big_q_dev;
-    DevArray<uint32_t> col_q32_dev;
-    DevArray<int8_t> col_label_dev;
-    DevArray<uint16_t> col_wig_dev, tbc_dev;      // ATTPC_COLUMNS_PACKED: wiggle, rows per (event, time bucket)
-    PinnedArray<uint16_t> col_wig_host, tbc_host;
-    PinnedArray<int16_t> col_pad_host;
-    PinnedArray<uint32_t> col_tbq_host;
-    PinnedArray<int64_t> col_q_host, big_rows_host, big_q_host;
-    PinnedArray<uint32_t> col_q32_host;
+    // outputs.  The row-indexed ones are sinks, reserved and copied through the lists of an OutputPlan; every sink a
+    // call uses holds out_rows rows (the Spyral rows of an event are a subset of its cloud rows).
+    int64_t out_rows = 0;
+    Sink<double, 3> cloud;
+    Sink<int64_t> labels;
+    Sink<int16_t> col_pad;
+    Sink<uint32_t> col_tbq, col_q32;
+    Sink<int64_t> col_q;
+    Sink<int8_t> col_label;
+    Sink<uint16_t> col_wig;  // ATTPC_COLUMNS_PACKED: wiggle
+    Sink<double, 8> rows;    // thresholded, z-ordered Spyral rows
+    Sink<int64_t> row_labels;
+    Sink<int16_t> rcol_pad;  // ... as typed columns (ATTPC_SPYRAL_COLUMNS)
+    Sink<uint32_t> rcol_tbq, rcol_elo;
+    Sink<uint16_t> rcol_ehi;
+    Sink<int8_t> rcol_label;
+    DevArray<int64_t> offsets_dev, row_offsets_dev, big_rows_dev, big_q_dev;
+    PinnedArray<int64_t> offsets_host, row_offsets_host, big_rows_host, big_q_host;
+    DevArray<uint16_t> tbc_dev;  // ATTPC_COLUMNS_PACKED: rows per (event, time bucket)
+    PinnedArray<uint16_t> tbc_host;
     bool q32_off = false;  // sticky: a call overflowed the exception list (heavy ions): later calls copy int64 directly
-    PinnedArray<int8_t> col_label_host;
-    bool columns = false;  // sticky: once a call asked for columns the buffers are kept in step with the others
-    DevArray<int64_t> offsets_dev, labels_dev, row_offsets_dev, row_labels_dev;
-    DevArray<double> cloud_dev, rows_dev;
     DevArray<unsigned> row_kept;
     DevArray<uint64_t> row_sort_keys;
     DevArray<uint32_t> row_sort_idx;
-    // thresholded, z-ordered Spyral rows as typed columns (ATTPC_SPYRAL_COLUMNS)
-    DevArray<int16_t> rcol_pad_dev;
-    DevArray<uint32_t> rcol_tbq_dev, rcol_elo_dev;
-    DevArray<uint16_t> rcol_ehi_dev;
-    DevArray<int8_t> rcol_label_dev;
-    PinnedArray<int16_t> rcol_pad_host;
-    PinnedArray<uint32_t> rcol_tbq_host, rcol_elo_host;
-    PinnedArray<uint16_t> rcol_ehi_host;
-    PinnedArray<int8_t> rcol_label_host;
-    PinnedArray<int64_t> offsets_host, labels_host, row_offsets_host, row_labels_host;
-    PinnedArray<double> cloud_host, rows_host;
 
     std::vector<cudaEvent_t> events;
     size_t events_used = 0;
     int launches = 0;
+
+    ~AttpcSim() {  // the arrays free themselves after this
+        for (cudaStream_t s : {stream, stream_t, stream_c})
+            if (s) cudaStreamSynchronize(s);
+        for (auto e : events) cudaEventDestroy(e);
+        for (auto e : sync_events) cudaEventDestroy(e);
+        for (cudaStream_t s : {stream, stream_t, stream_c})
+            if (s) cudaStreamDestroy(s);
+    }
 
     int fail(int code, const char* fmt, ...) {
         char buf[512];
@@ -299,25 +346,6 @@ int ensure_work_buffers(AttpcSim* sim, int64_t launch_events, int32_t ranks, int
     CU(sim->csr_total.reserve(3));  // cloud rows, electron counts >= 2^32, Spyral rows
     CU(sim->csr_host.reserve(3));
     CU(sim->chunk_totals.reserve(2 * (n_groups + 1)));
-    return ATTPC_OK;
-}
-
-int ensure_out_buffers(AttpcSim* sim, int64_t n_events, int64_t n_points, bool keep) {
-    CU(sim->offsets_dev.reserve(n_events + 1, keep, sim->stream));
-    CU(sim->kept.reserve(n_events + 1, keep, sim->stream));
-    CU(sim->cloud_dev.reserve(n_points * 3, keep, sim->stream));
-    CU(sim->labels_dev.reserve(n_points, keep, sim->stream));
-    if (sim->columns) {
-        CU(sim->col_pad_dev.reserve(sim->labels_dev.n, keep, sim->stream));
-        CU(sim->col_tbq_dev.reserve(sim->labels_dev.n, keep, sim->stream));
-        CU(sim->col_q_dev.reserve(sim->labels_dev.n, keep, sim->stream));
-        CU(sim->col_q32_dev.reserve(sim->labels_dev.n, keep, sim->stream));
-        CU(sim->big_rows_dev.reserve(ATTPC_BIG_CAP));
-        CU(sim->big_q_dev.reserve(ATTPC_BIG_CAP));
-        CU(sim->col_label_dev.reserve(sim->labels_dev.n, keep, sim->stream));
-        CU(sim->col_wig_dev.reserve(sim->labels_dev.n, keep, sim->stream));
-        CU(sim->tbc_dev.reserve((n_events + 1) * NUM_TB, keep, sim->stream));
-    }
     return ATTPC_OK;
 }
 
@@ -519,52 +547,31 @@ float sum_ms(const std::vector<std::pair<cudaEvent_t, cudaEvent_t>>& marks) {
     return total;
 }
 
-// Buffers of the Spyral passes for clouds of up to n_points rows; `typed`: the typed-column sink as well.
-int ensure_spyral_buffers(AttpcSim* sim, int64_t n_events, int64_t n_points, bool typed, bool f64_rows) {
-    n_points = std::max<int64_t>(1, n_points);
-    CU(sim->row_kept.reserve(n_events + 1));
-    CU(sim->row_offsets_dev.reserve(n_events + 1));
-    CU(sim->row_sort_keys.reserve(n_points * 2));
-    CU(sim->row_sort_idx.reserve(n_points * 2));
-    if (f64_rows) {
-        CU(sim->rows_dev.reserve(n_points * 8));
-        CU(sim->row_labels_dev.reserve(n_points));
-    }
-    if (typed) {
-        CU(sim->rcol_pad_dev.reserve(n_points));
-        CU(sim->rcol_tbq_dev.reserve(n_points));
-        CU(sim->rcol_elo_dev.reserve(n_points));
-        CU(sim->rcol_ehi_dev.reserve(n_points));
-        CU(sim->rcol_label_dev.reserve(n_points));
-    }
-    return ATTPC_OK;
-}
-
 SpyralArgs spyral_args(AttpcSim* sim, int64_t first, int64_t n_events, bool typed, bool keep_all, const Counters* ctr) {
     SpyralArgs sa;
     memset(&sa, 0, sizeof sa);
     sa.offsets = sim->offsets_dev.p;
-    sa.cloud = sim->cloud_dev.p;
-    sa.labels = sim->labels_dev.p;
+    sa.cloud = sim->cloud.d();
+    sa.labels = sim->labels.d();
     sa.n_events = n_events;
     sa.first = first;
     sa.total = sim->csr_total.p + 2;
     sa.scratch_rows = sim->row_sort_keys.n / 2;
     sa.ctr = ctr;
-    sa.cloud_cap = std::min<int64_t>(sim->labels_dev.n, sa.scratch_rows);
+    sa.cloud_cap = std::min<int64_t>(sim->labels.dev.n / sim->labels.row_bytes, sa.scratch_rows);
     sa.kept = sim->row_kept.p;
     sa.row_offsets = sim->row_offsets_dev.p;
-    sa.rows = sim->rows_dev.p;
-    sa.row_labels = sim->row_labels_dev.p;
+    sa.rows = sim->rows.d();
+    sa.row_labels = sim->row_labels.d();
     sa.sort_keys = sim->row_sort_keys.p;
     sa.sort_idx = sim->row_sort_idx.p;
     sa.keep_all = keep_all ? 1 : 0;
     if (typed) {
-        sa.out_pad = sim->rcol_pad_dev.p;
-        sa.out_tb_q16 = sim->rcol_tbq_dev.p;
-        sa.out_e_lo = sim->rcol_elo_dev.p;
-        sa.out_e_hi = sim->rcol_ehi_dev.p;
-        sa.out_label = sim->rcol_label_dev.p;
+        sa.out_pad = sim->rcol_pad.d();
+        sa.out_tb_q16 = sim->rcol_tbq.d();
+        sa.out_e_lo = sim->rcol_elo.d();
+        sa.out_e_hi = sim->rcol_ehi.d();
+        sa.out_label = sim->rcol_label.d();
     }
     return sa;
 }
@@ -580,39 +587,6 @@ int launch_spyral(AttpcSim* sim, const SpyralArgs& sa) {
     spyral_rows_kernel<<<(unsigned)sa.n_events, 256, smem, sim->stream>>>(sim->P, sa);
     sim->launches += 3;
     CU(cudaGetLastError());
-    return ATTPC_OK;
-}
-
-// attpc_convert_to_spyral: the whole (host-supplied) cloud in one pass, float64 rows back to the host.
-int run_spyral(AttpcSim* sim, int64_t n_events, int64_t n_points, AttpcResult* res, bool copy_host,
-               bool keep_all = false) {
-    int rc = ensure_spyral_buffers(sim, n_events, n_points, false, true);
-    if (rc) return rc;
-    CU(sim->csr_total.reserve(3));
-    CU(cudaMemsetAsync(sim->csr_total.p + 2, 0, sizeof(unsigned long long), sim->stream));
-    CU(cudaMemsetAsync(sim->row_offsets_dev.p, 0, sizeof(int64_t), sim->stream));
-    rc = launch_spyral(sim, spyral_args(sim, 0, n_events, false, keep_all, nullptr));
-    if (rc) return rc;
-    CU(sim->row_offsets_host.reserve(n_events + 1));
-    CU(cudaMemcpyAsync(sim->row_offsets_host.p, sim->row_offsets_dev.p, (size_t)(n_events + 1) * sizeof(int64_t),
-                       cudaMemcpyDeviceToHost, sim->stream));
-    CU(cudaStreamSynchronize(sim->stream));
-    const int64_t n_rows = sim->row_offsets_host.p[n_events];
-    res->n_rows = n_rows;
-    res->row_offsets = sim->row_offsets_host.p;
-    if (copy_host) {
-        CU(sim->rows_host.reserve(std::max<int64_t>(1, n_rows) * 8));
-        CU(sim->row_labels_host.reserve(std::max<int64_t>(1, n_rows)));
-        if (n_rows > 0) {
-            CU(cudaMemcpyAsync(sim->rows_host.p, sim->rows_dev.p, (size_t)n_rows * 8 * sizeof(double),
-                               cudaMemcpyDeviceToHost, sim->stream));
-            CU(cudaMemcpyAsync(sim->row_labels_host.p, sim->row_labels_dev.p, (size_t)n_rows * sizeof(int64_t),
-                               cudaMemcpyDeviceToHost, sim->stream));
-        }
-        CU(cudaStreamSynchronize(sim->stream));
-        res->rows = sim->rows_host.p;
-        res->row_labels = sim->row_labels_host.p;
-    }
     return ATTPC_OK;
 }
 
@@ -632,6 +606,299 @@ struct LaunchPlan {
     ReplayUniforms uniforms{nullptr, nullptr, nullptr};
 };
 
+// What one call writes and returns, derived from its flags once.
+struct OutputPlan {
+    bool copy_host = false;
+    bool use_columns = false, use_q32 = false, use_packed = false;
+    bool spy_cols = false, spy_rows = false, spy = false, spy_fused = false;
+    bool copy_cloud = false, want_cloud = false;
+    struct Use {
+        RowSink* sink;
+        bool to_host;  // copied to its pinned mirror; otherwise it stays on the device
+    };
+    std::vector<Use> cloud_rows;   // the sinks the call writes, indexed by cloud row, in the order they are copied
+    std::vector<Use> spyral_rows;  // ... indexed by Spyral row
+};
+
+OutputPlan plan_outputs(AttpcSim* sim, const LaunchPlan& plan, uint32_t flags) {
+    OutputPlan op;
+    op.copy_host = !(flags & ATTPC_SKIP_HOST_COPY);
+    op.use_columns = op.copy_host && (flags & ATTPC_COLUMNS);
+    op.use_q32 = op.use_columns && (flags & ATTPC_COLUMNS32) && !sim->q32_off;
+    // packed columns: pad ids and track ranks share 16 bits, the library's own 16-bit wiggle, masked time buckets
+    op.use_packed = op.use_columns && (flags & ATTPC_COLUMNS_PACKED) && !plan.replay && !(flags & ATTPC_KEEP_ALL_TB) &&
+                    sim->P.n_pads <= (1 << 14) && plan.n_tracks_per_event <= 4;
+    op.spy_cols = (flags & ATTPC_SPYRAL_COLUMNS) != 0;               // Spyral rows as typed columns
+    op.spy_rows = (flags & ATTPC_SPYRAL_ROWS) != 0 && !op.spy_cols;  // ... as float64 [M, 8]
+    op.spy = op.spy_cols || op.spy_rows;
+    op.copy_cloud = op.copy_host && !op.use_columns && !((flags & ATTPC_SKIP_CLOUD_COPY) && op.spy);
+    // the float64 rows on the device: the product of a device-resident call, the input of the Spyral passes
+    // (replayed 53-bit uniforms and unmasked time buckets: separate passes over the float64 cloud)
+    op.spy_fused = op.spy && !plan.replay && !(flags & ATTPC_KEEP_ALL_TB);
+    // nobody reads the float64 rows when the call returns typed columns, or only the Spyral rows, to the host
+    const bool cloud_unread = op.copy_host && (op.use_columns || ((flags & ATTPC_SKIP_CLOUD_COPY) && op.spy));
+    op.want_cloud = !cloud_unread || (op.spy && !op.spy_fused);
+    if (op.want_cloud) op.cloud_rows = {{&sim->cloud, op.copy_cloud}, {&sim->labels, op.copy_cloud}};
+    if (op.use_columns) {
+        op.cloud_rows.push_back({&sim->col_pad, true});
+        if (op.use_packed) op.cloud_rows.push_back({&sim->col_wig, true});
+        else op.cloud_rows.push_back({&sim->col_tbq, true});
+        if (op.use_q32) op.cloud_rows.push_back({&sim->col_q32, true});
+        else op.cloud_rows.push_back({&sim->col_q, true});
+        if (!op.use_packed) op.cloud_rows.push_back({&sim->col_label, true});
+    }
+    const bool h = op.copy_host;
+    if (op.spy_rows) op.spyral_rows = {{&sim->rows, h}, {&sim->row_labels, h}};
+    if (op.spy_cols)
+        op.spyral_rows = {{&sim->rcol_pad, h}, {&sim->rcol_tbq, h}, {&sim->rcol_elo, h}, {&sim->rcol_ehi, h},
+                          {&sim->rcol_label, h}};
+    return op;
+}
+
+// Room for n_events events and `rows` cloud rows in the outputs of `op`.  `keep`: the rows written so far survive, on
+// the device and on the host (regrowth after an output overflow).  The pinned mirrors are sized like the device
+// arrays: pinning is slow, so they are (re)allocated only when those grow.
+int reserve_outputs(AttpcSim* sim, const OutputPlan& op, int64_t n_events, int64_t rows, bool keep) {
+    cudaStream_t s = sim->stream;
+    CU(sim->offsets_dev.reserve(n_events + 1, keep, s));
+    CU(sim->kept.reserve(n_events + 1, keep, s));
+    if (op.copy_host) CU(sim->offsets_host.reserve(sim->offsets_dev.n, keep));
+    if (op.use_packed) {
+        CU(sim->tbc_dev.reserve((n_events + 1) * NUM_TB, keep, s));
+        CU(sim->tbc_host.reserve(sim->tbc_dev.n, keep));
+    }
+    if (op.use_q32) {
+        CU(sim->big_rows_dev.reserve(ATTPC_BIG_CAP));
+        CU(sim->big_q_dev.reserve(ATTPC_BIG_CAP));
+    }
+    if (op.spy) {
+        CU(sim->row_kept.reserve(n_events + 1));
+        CU(sim->row_offsets_dev.reserve(n_events + 1));
+        if (op.copy_host) CU(sim->row_offsets_host.reserve(n_events + 1, keep));
+        CU(sim->row_sort_keys.reserve(rows * 2));  // scratch of the Spyral passes: nothing to keep
+        CU(sim->row_sort_idx.reserve(rows * 2));
+    }
+    for (const auto* list : {&op.cloud_rows, &op.spyral_rows})
+        for (const OutputPlan::Use& u : *list) {
+            CU(u.sink->reserve(rows, keep, s));
+            if (u.to_host) CU(u.sink->reserve_host(rows, keep));
+        }
+    sim->out_rows = std::max(sim->out_rows, rows);
+    return ATTPC_OK;
+}
+
+// How far the host copies have got: events of the current launch whose offsets are final there, cloud rows and
+// Spyral rows of the call.
+struct CopyMark {
+    int64_t events;
+    unsigned long long cloud, spyral;
+};
+
+// Enqueues on the copy stream what became final between `from` and `to` in the launch whose first event is b0.
+int copy_outputs(AttpcSim* sim, const OutputPlan& op, int64_t b0, const CopyMark& from, const CopyMark& to) {
+    cudaStream_t C = sim->stream_c;
+    const int64_t first_off = (b0 + from.events == 0) ? 0 : b0 + from.events + 1;  // the entry before is there already
+    const int64_t end_off = b0 + to.events + 1;
+    if (end_off > first_off) {
+        CU(cudaMemcpyAsync(sim->offsets_host.p + first_off, sim->offsets_dev.p + first_off,
+                           (size_t)(end_off - first_off) * sizeof(int64_t), cudaMemcpyDeviceToHost, C));
+        if (op.spy)
+            CU(cudaMemcpyAsync(sim->row_offsets_host.p + first_off, sim->row_offsets_dev.p + first_off,
+                               (size_t)(end_off - first_off) * sizeof(int64_t), cudaMemcpyDeviceToHost, C));
+    }
+    if (op.use_packed && to.events > from.events)
+        CU(cudaMemcpyAsync(sim->tbc_host.p + (b0 + from.events) * NUM_TB, sim->tbc_dev.p + (b0 + from.events) * NUM_TB,
+                           (size_t)(to.events - from.events) * NUM_TB * sizeof(uint16_t), cudaMemcpyDeviceToHost, C));
+    const int64_t r_new = (int64_t)(to.spyral - from.spyral);
+    for (const OutputPlan::Use& u : op.spyral_rows)
+        if (u.to_host && r_new > 0) CU(u.sink->copy_to_host((int64_t)from.spyral, r_new, C));
+    const int64_t n_new = (int64_t)(to.cloud - from.cloud);
+    for (const OutputPlan::Use& u : op.cloud_rows)
+        if (u.to_host && n_new > 0) CU(u.sink->copy_to_host((int64_t)from.cloud, n_new, C));
+    return ATTPC_OK;
+}
+
+// The finalize kernels' arguments for the launch whose first event is b0.
+FinalizeArgs finalize_args(AttpcSim* sim, const LaunchPlan& plan, const OutputPlan& op, uint32_t flags, int64_t b0) {
+    FinalizeArgs fa;
+    memset(&fa, 0, sizeof fa);
+    fa.seed = plan.seed;
+    fa.first_event = plan.first_event + b0;
+    fa.flags = flags;
+    fa.kept = sim->kept.p + b0;
+    fa.offsets = sim->offsets_dev.p + b0;
+    fa.cloud = op.want_cloud ? sim->cloud.d() : nullptr;  // typed columns only: the float64 rows are not written
+    fa.labels = op.want_cloud ? sim->labels.d() : nullptr;
+    fa.out_cap = sim->out_rows;
+    if (op.use_columns) {
+        fa.col_pad = sim->col_pad.d();
+        if (op.use_packed) {
+            fa.col_wiggle = sim->col_wig.d();
+            fa.tb_counts = sim->tbc_dev.p + b0 * NUM_TB;
+            fa.rank_shift = 14;
+        } else {
+            fa.col_tb_q16 = sim->col_tbq.d();
+            fa.col_label = sim->col_label.d();
+        }
+        if (op.use_q32) {
+            fa.col_electrons32 = sim->col_q32.d();
+            fa.big_rows = sim->big_rows_dev.p;
+            fa.big_electrons = sim->big_q_dev.p;
+            fa.big_count = sim->csr_total.p + 1;
+            fa.big_cap = sim->big_cap;
+        } else {
+            fa.col_electrons = sim->col_q.d();
+        }
+    }
+    if (op.spy_fused) {
+        fa.spyral = op.spy_cols ? 1u : 2u;
+        fa.row_kept = sim->row_kept.p + b0;
+        fa.row_offsets = sim->row_offsets_dev.p + b0;
+        if (op.spy_cols) {
+            fa.rcol_pad = sim->rcol_pad.d();
+            fa.rcol_tb_q16 = sim->rcol_tbq.d();
+            fa.rcol_e_lo = sim->rcol_elo.d();
+            fa.rcol_e_hi = sim->rcol_ehi.d();
+            fa.rcol_label = sim->rcol_label.d();
+        } else {
+            fa.rows = sim->rows.d();
+            fa.row_labels = sim->row_labels.d();
+        }
+    }
+    fa.replay = plan.uniforms;
+    if (fa.replay.offsets) fa.replay.offsets += b0;
+    fa.n_tracks_per_event = plan.n_tracks_per_event;
+    if (plan.replay) {
+        fa.label_of_event_rank = plan.label_of_event_rank_dev;
+    } else {
+        for (int t = 0; t < plan.n_tracks_per_event; ++t) fa.label_of_rank[t] = plan.track_nucleus[t];
+    }
+    return fa;
+}
+
+// Grows what a launch overflowed before it is redone.  The output rows of earlier launches are kept, on the device
+// and on the host.
+int grow_buffers(AttpcSim* sim, const Counters& now, const OutputPlan& op, int64_t n_events, int64_t work_events,
+                 int32_t ranks, int64_t table_groups) {
+    CU(cudaStreamSynchronize(sim->stream_t));  // the next launch's track kernel may be using buffers we are about to free
+    CU(cudaStreamSynchronize(sim->stream_c));
+    if (now.overflow_sub) {  // (overflow_points is raised with it: the point lists themselves were complete)
+        if (sim->sub_cap >= (1LL << 30)) return sim->fail(ATTPC_E_CAPACITY, "a group needs > 2^30 sub-points");
+        sim->sub_cap *= 2;
+        sim->geom.release(); sim->rec.release();
+        sim->unit_event.release(); sim->unit_first.release(); sim->unit_count.release();
+        sim->unit_order.release();
+    } else if (now.overflow_points) {
+        sim->group_point_cap *= 2;
+        for (auto& s2 : sim->slot) s2.release_points();
+        sim->geom.release(); sim->rec.release();
+        sim->unit_event.release(); sim->unit_first.release(); sim->unit_count.release();
+        sim->unit_order.release();
+    }
+    if (now.overflow_hash) {
+        if (sim->hash_cap >= (1 << 20)) return sim->fail(ATTPC_E_CAPACITY, "event needs > 2^20 hash slots");
+        sim->hash_cap *= 2;
+        sim->hash.release();
+        sim->sort_items.release();
+        sim->staged.release();
+    }
+    if (now.overflow_out) {
+        const int64_t rows = std::max<int64_t>(sim->out_rows * 2, (int64_t)sim->csr_host.p[0] + (1 << 20));
+        const int rc = reserve_outputs(sim, op, n_events, rows, true);
+        if (rc) return rc;
+    }
+    return ensure_work_buffers(sim, work_events, ranks, table_groups);
+}
+
+void add_counters(Counters& totals, const Counters& now) {
+    totals.traj_points += now.traj_points;
+    totals.active_points += now.active_points;
+    totals.primary_electrons += now.primary_electrons;
+    totals.deposits += now.deposits;
+    totals.keys += now.keys;
+    totals.probes += now.probes;
+    totals.flushes += now.flushes;
+    totals.rk_steps += now.rk_steps;
+    totals.rk_rejects += now.rk_rejects;
+    totals.max_track_passes = std::max(totals.max_track_passes, now.max_track_passes);
+}
+
+// The counters of a finished call and where its outputs are: `done` holds its events, cloud rows and Spyral rows,
+// n_big its electron counts >= 2^32.
+int publish_result(AttpcSim* sim, const OutputPlan& op, const Counters& totals, int retries, const CopyMark& done,
+                   unsigned long long n_big, AttpcResult* res) {
+    res->n_points = (int64_t)done.cloud;
+    res->offsets_dev = sim->offsets_dev.p;
+    if (op.want_cloud) {
+        res->cloud_dev = sim->cloud.d();
+        res->labels_dev = sim->labels.d();
+    }
+    res->n_trajectory_points = (int64_t)totals.traj_points;
+    res->n_active_points = (int64_t)totals.active_points;
+    res->n_primary_electrons = (int64_t)totals.primary_electrons;
+    res->n_deposits = (int64_t)totals.deposits;
+    res->n_keys = (int64_t)totals.keys;
+    res->n_hash_probes = (int64_t)totals.probes;
+    res->n_table_flushes = (int64_t)totals.flushes;
+    res->n_rk_steps = (int64_t)totals.rk_steps;
+    res->n_rk_rejects = (int64_t)totals.rk_rejects;
+    res->max_track_passes = (int64_t)totals.max_track_passes;
+    res->n_retries = retries;
+    if (op.spy) res->n_rows = (int64_t)done.spyral;
+    if (!op.copy_host) return ATTPC_OK;
+    if (done.events == 0) {  // no launch copied the leading offsets
+        const int rc = copy_outputs(sim, op, 0, CopyMark{0, 0, 0}, CopyMark{0, 0, 0});
+        if (rc) return rc;
+    }
+    cudaStream_t C = sim->stream_c;
+    res->offsets = sim->offsets_host.p;
+    if (op.copy_cloud) {
+        res->cloud = sim->cloud.h();
+        res->labels = sim->labels.h();
+    }
+    if (op.use_columns) {
+        res->col_pad = sim->col_pad.h();
+        if (op.use_packed) {
+            res->col_wiggle = sim->col_wig.h();
+            res->tb_counts = sim->tbc_host.p;
+            res->pad_rank_shift = 14;
+        } else {
+            res->col_tb_q16 = sim->col_tbq.h();
+            res->col_label = sim->col_label.h();
+        }
+        if (!op.use_q32) {
+            res->col_electrons = sim->col_q.h();
+        } else {
+            res->col_electrons32 = sim->col_q32.h();
+            res->n_big = (int64_t)n_big;
+            if (n_big > 0) {
+                CU(sim->big_rows_host.reserve((int64_t)n_big));
+                CU(sim->big_q_host.reserve((int64_t)n_big));
+                CU(cudaMemcpyAsync(sim->big_rows_host.p, sim->big_rows_dev.p, (size_t)n_big * sizeof(int64_t),
+                                   cudaMemcpyDeviceToHost, C));
+                CU(cudaMemcpyAsync(sim->big_q_host.p, sim->big_q_dev.p, (size_t)n_big * sizeof(int64_t),
+                                   cudaMemcpyDeviceToHost, C));
+                res->big_rows = sim->big_rows_host.p;
+                res->big_electrons = sim->big_q_host.p;
+            }
+        }
+    }
+    if (op.spy) {
+        res->row_offsets = sim->row_offsets_host.p;
+        if (op.spy_rows) {
+            res->rows = sim->rows.h();
+            res->row_labels = sim->row_labels.h();
+        } else {
+            res->row_col_pad = sim->rcol_pad.h();
+            res->row_col_tb_q16 = sim->rcol_tbq.h();
+            res->row_col_e_lo = sim->rcol_elo.h();
+            res->row_col_e_hi = sim->rcol_ehi.h();
+            res->row_col_label = sim->rcol_label.h();
+        }
+    }
+    return ATTPC_OK;
+}
+
 // Shared driver of attpc_simulate / attpc_simulate_dev / attpc_simulate_replay.
 //
 // Three streams: T runs the (latency-bound, few-warp) track kernel of launch i+1 while G runs the deposit and
@@ -645,25 +912,9 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
     sim->launches = 0;
     res->n_events = n_events;
     res->ms_h2d = ms_h2d;
-    const bool copy_host = !(flags & ATTPC_SKIP_HOST_COPY);
-    const bool use_columns = copy_host && (flags & ATTPC_COLUMNS);
-    const bool use_q32 = use_columns && (flags & ATTPC_COLUMNS32) && !sim->q32_off;
-    // packed columns: pad ids and track ranks share 16 bits, the library's own 16-bit wiggle, masked time buckets
-    const bool use_packed = use_columns && (flags & ATTPC_COLUMNS_PACKED) && !plan.replay &&
-                            !(flags & ATTPC_KEEP_ALL_TB) && sim->P.n_pads <= (1 << 14) && plan.n_tracks_per_event <= 4;
-    const bool spy_cols = (flags & ATTPC_SPYRAL_COLUMNS) != 0;            // Spyral rows as typed columns
-    const bool spy_rows = (flags & ATTPC_SPYRAL_ROWS) != 0 && !spy_cols;  // ... as float64 [M, 8]
-    const bool spy = spy_cols || spy_rows;
-    const bool copy_cloud = copy_host && !use_columns && !((flags & ATTPC_SKIP_CLOUD_COPY) && spy);
-    // the float64 rows on the device: the product of a device-resident call, the input of the Spyral passes
-    // (replayed 53-bit uniforms and unmasked time buckets: separate passes over the float64 cloud)
-    const bool spy_fused = spy && !plan.replay && !(flags & ATTPC_KEEP_ALL_TB);
-    // nobody reads the float64 rows when the call returns typed columns, or only the Spyral rows, to the host
-    const bool cloud_unread = copy_host && (use_columns || ((flags & ATTPC_SKIP_CLOUD_COPY) && spy));
-    const bool want_cloud = !cloud_unread || (spy && !spy_fused);
-    if (use_columns) sim->columns = true;
-    int64_t out_cap = std::max<int64_t>(sim->labels_dev.n, std::max<int64_t>(n_events * 2048, 1 << 20));
-    int rc = ensure_out_buffers(sim, n_events, out_cap, false);
+    const OutputPlan op = plan_outputs(sim, plan, flags);
+    int rc = reserve_outputs(sim, op, n_events,
+                             std::max<int64_t>(sim->out_rows, std::max<int64_t>(n_events * 2048, 1 << 20)), false);
     if (rc) return rc;
     // big launches: the latency-bound track kernel wants many tracks in flight.  When rows go to the host they are
     // copied in chunks of a few groups while the following groups are still being computed.
@@ -672,50 +923,14 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
         std::max<int>(1, (int)((sim->copy_launch_events + sim->group_events - 1) / sim->group_events));
     const int32_t ranks = std::max<int32_t>(1, plan.n_tracks_per_event);
     // a call that copies its rows to the host works in chunks of a few groups: its engine needs an eighth of the memory
-    const int64_t table_groups = copy_host ? groups_per_chunk : sim->chunk_groups;
-    rc = ensure_work_buffers(sim, std::min<int64_t>(std::max<int64_t>(n_events, 1), launch_cap), ranks, table_groups);
+    const int64_t table_groups = op.copy_host ? groups_per_chunk : sim->chunk_groups;
+    const int64_t work_events = std::min<int64_t>(std::max<int64_t>(n_events, 1), launch_cap);
+    rc = ensure_work_buffers(sim, work_events, ranks, table_groups);
     if (rc) return rc;
-    if (copy_host) CU(sim->offsets_host.reserve(sim->offsets_dev.n));
-    if (copy_cloud) {  // pinned mirrors are sized like the device buffers: (re)allocated only when those grow
-        CU(sim->cloud_host.reserve(sim->cloud_dev.n));
-        CU(sim->labels_host.reserve(sim->labels_dev.n));
-    }
-    if (use_columns) {
-        CU(sim->col_pad_host.reserve(sim->labels_dev.n));
-        CU(sim->col_tbq_host.reserve(sim->labels_dev.n));
-        if (use_q32) CU(sim->col_q32_host.reserve(sim->labels_dev.n));
-        else CU(sim->col_q_host.reserve(sim->labels_dev.n));
-        CU(sim->col_label_host.reserve(sim->labels_dev.n));
-        if (use_packed) {
-            CU(sim->col_wig_host.reserve(sim->labels_dev.n));
-            CU(sim->tbc_host.reserve(sim->tbc_dev.n));
-        }
-    }
-    auto reserve_spyral = [&](bool keep) -> int {  // the rows of an event are a subset of its cloud points
-        int r = ensure_spyral_buffers(sim, n_events, sim->labels_dev.n, spy_cols, spy_rows);
-        if (r) return r;
-        if (!copy_host) return ATTPC_OK;
-        CU(sim->row_offsets_host.reserve(n_events + 1, keep));
-        if (spy_rows) {
-            CU(sim->rows_host.reserve(sim->labels_dev.n * 8, keep));
-            CU(sim->row_labels_host.reserve(sim->labels_dev.n, keep));
-        } else {
-            CU(sim->rcol_pad_host.reserve(sim->labels_dev.n, keep));
-            CU(sim->rcol_tbq_host.reserve(sim->labels_dev.n, keep));
-            CU(sim->rcol_elo_host.reserve(sim->labels_dev.n, keep));
-            CU(sim->rcol_ehi_host.reserve(sim->labels_dev.n, keep));
-            CU(sim->rcol_label_host.reserve(sim->labels_dev.n, keep));
-        }
-        return ATTPC_OK;
-    };
-    if (spy) {
-        rc = reserve_spyral(false);
-        if (rc) return rc;
-    }
-    const SpyralPass spyral_pass{spy_cols};
+    const SpyralPass spyral_pass{op.spy_cols};
     cudaStream_t G = sim->stream, T = sim->stream_t, C = sim->stream_c;
     CU(cudaMemsetAsync(sim->csr_total.p, 0, 3 * sizeof(unsigned long long), G));
-    if (spy) CU(cudaMemsetAsync(sim->row_offsets_dev.p, 0, sizeof(int64_t), G));
+    if (op.spy) CU(cudaMemsetAsync(sim->row_offsets_dev.p, 0, sizeof(int64_t), G));
     CU(cudaMemsetAsync(sim->offsets_dev.p, 0, sizeof(int64_t), G));
     cudaEvent_t t_begin = sim->mark(G);
     CU(cudaStreamWaitEvent(T, t_begin, 0));
@@ -727,7 +942,7 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
     std::vector<int64_t> launch_begin;
     {
         int64_t at = 0;
-        if (copy_host && !plan.replay && n_events > 2 * (int64_t)sim->group_events && launch_cap > sim->group_events) {
+        if (op.copy_host && !plan.replay && n_events > 2 * (int64_t)sim->group_events && launch_cap > sim->group_events) {
             launch_begin.push_back(0);
             at = sim->group_events;
         }
@@ -806,65 +1021,13 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
             rc = enqueue_track(next_track++);
             if (rc) return rc;
         }
-        FinalizeArgs fa;
-        memset(&fa, 0, sizeof fa);
-        fa.seed = plan.seed;
-        fa.first_event = plan.first_event + b0;
-        fa.flags = flags;
-        fa.kept = sim->kept.p + b0;
-        fa.offsets = sim->offsets_dev.p + b0;
-        fa.cloud = want_cloud ? sim->cloud_dev.p : nullptr;  // typed columns only: the float64 rows are not written
-        fa.labels = want_cloud ? sim->labels_dev.p : nullptr;
-        fa.out_cap = sim->labels_dev.n;
-        if (use_columns) {
-            fa.col_pad = sim->col_pad_dev.p;
-            if (use_packed) {
-                fa.col_wiggle = sim->col_wig_dev.p;
-                fa.tb_counts = sim->tbc_dev.p + b0 * NUM_TB;
-                fa.rank_shift = 14;
-            } else {
-                fa.col_tb_q16 = sim->col_tbq_dev.p;
-                fa.col_label = sim->col_label_dev.p;
-            }
-            if (use_q32) {
-                fa.col_electrons32 = sim->col_q32_dev.p;
-                fa.big_rows = sim->big_rows_dev.p;
-                fa.big_electrons = sim->big_q_dev.p;
-                fa.big_count = sim->csr_total.p + 1;
-                fa.big_cap = sim->big_cap;
-            } else {
-                fa.col_electrons = sim->col_q_dev.p;
-            }
-        }
-        if (spy_fused) {
-            fa.spyral = spy_cols ? 1u : 2u;
-            fa.row_kept = sim->row_kept.p + b0;
-            fa.row_offsets = sim->row_offsets_dev.p + b0;
-            if (spy_cols) {
-                fa.rcol_pad = sim->rcol_pad_dev.p;
-                fa.rcol_tb_q16 = sim->rcol_tbq_dev.p;
-                fa.rcol_e_lo = sim->rcol_elo_dev.p;
-                fa.rcol_e_hi = sim->rcol_ehi_dev.p;
-                fa.rcol_label = sim->rcol_label_dev.p;
-            } else {
-                fa.rows = sim->rows_dev.p;
-                fa.row_labels = sim->row_labels_dev.p;
-            }
-        }
-        fa.replay = plan.uniforms;
-        if (fa.replay.offsets) fa.replay.offsets += b0;
-        fa.n_tracks_per_event = plan.n_tracks_per_event;
-        if (plan.replay) {
-            fa.label_of_event_rank = plan.label_of_event_rank_dev;
-        } else {
-            for (int t = 0; t < plan.n_tracks_per_event; ++t) fa.label_of_rank[t] = plan.track_nucleus[t];
-        }
+        const FinalizeArgs fa = finalize_args(sim, plan, op, flags, b0);
         CU(cudaStreamWaitEvent(G, track_done[i], 0));
         const size_t dep_before = dep_marks.size(), fin_before = fin_marks.size(), copy_before = copy_marks.size();
         const size_t ord_before = ord_marks.size();
         std::vector<ChunkFence> fences;
         rc = run_groups(sim, nb, fa, which, ord_marks, dep_marks, fin_marks, groups_per_chunk,
-                        copy_host ? &fences : nullptr, spy && !spy_fused ? &spyral_pass : nullptr, b0);
+                        op.copy_host ? &fences : nullptr, op.spy && !op.spy_fused ? &spyral_pass : nullptr, b0);
         if (rc) return rc;
         publish_kernel<<<1, 1, 0, G>>>(ls.counters.p, sim->csr_total.p, ls.counters_host.p, sim->csr_host.p);
         sim->launches += 1;
@@ -874,81 +1037,21 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
             if (rc) return rc;
         }
         // rows of finished chunks go home while the later groups (and the next launch's tracks) compute
-        unsigned long long copied = csr_before, rows_copied = rows_before;
-        int64_t copied_events = 0;  // events of this launch whose offsets are on the host
-        auto copy_rows = [&](unsigned long long upto, unsigned long long rows_upto, int64_t upto_event) -> int {
+        CopyMark copied{0, csr_before, rows_before};  // events of this launch, rows of the call, on the host
+        auto copy_rows = [&](const CopyMark& upto) -> int {
             cudaEvent_t c0 = sim->mark(C);
-            const int64_t first_off = (b0 + copied_events == 0) ? 0 : b0 + copied_events + 1;
-            const int64_t end_off = b0 + upto_event + 1;
-            if (end_off > first_off) {
-                CU(cudaMemcpyAsync(sim->offsets_host.p + first_off, sim->offsets_dev.p + first_off,
-                                   (size_t)(end_off - first_off) * sizeof(int64_t), cudaMemcpyDeviceToHost, C));
-                if (spy)
-                    CU(cudaMemcpyAsync(sim->row_offsets_host.p + first_off, sim->row_offsets_dev.p + first_off,
-                                       (size_t)(end_off - first_off) * sizeof(int64_t), cudaMemcpyDeviceToHost, C));
-            }
-            if (use_packed && upto_event > copied_events)
-                CU(cudaMemcpyAsync(sim->tbc_host.p + (b0 + copied_events) * NUM_TB,
-                                   sim->tbc_dev.p + (b0 + copied_events) * NUM_TB,
-                                   (size_t)(upto_event - copied_events) * NUM_TB * sizeof(uint16_t),
-                                   cudaMemcpyDeviceToHost, C));
-            const int64_t r_new = (int64_t)(rows_upto - rows_copied);
-            if (r_new > 0 && spy_rows) {
-                CU(cudaMemcpyAsync(sim->rows_host.p + rows_copied * 8, sim->rows_dev.p + rows_copied * 8,
-                                   (size_t)r_new * 8 * sizeof(double), cudaMemcpyDeviceToHost, C));
-                CU(cudaMemcpyAsync(sim->row_labels_host.p + rows_copied, sim->row_labels_dev.p + rows_copied,
-                                   (size_t)r_new * sizeof(int64_t), cudaMemcpyDeviceToHost, C));
-            }
-            if (r_new > 0 && spy_cols) {
-                CU(cudaMemcpyAsync(sim->rcol_pad_host.p + rows_copied, sim->rcol_pad_dev.p + rows_copied,
-                                   (size_t)r_new * sizeof(int16_t), cudaMemcpyDeviceToHost, C));
-                CU(cudaMemcpyAsync(sim->rcol_tbq_host.p + rows_copied, sim->rcol_tbq_dev.p + rows_copied,
-                                   (size_t)r_new * sizeof(uint32_t), cudaMemcpyDeviceToHost, C));
-                CU(cudaMemcpyAsync(sim->rcol_elo_host.p + rows_copied, sim->rcol_elo_dev.p + rows_copied,
-                                   (size_t)r_new * sizeof(uint32_t), cudaMemcpyDeviceToHost, C));
-                CU(cudaMemcpyAsync(sim->rcol_ehi_host.p + rows_copied, sim->rcol_ehi_dev.p + rows_copied,
-                                   (size_t)r_new * sizeof(uint16_t), cudaMemcpyDeviceToHost, C));
-                CU(cudaMemcpyAsync(sim->rcol_label_host.p + rows_copied, sim->rcol_label_dev.p + rows_copied,
-                                   (size_t)r_new * sizeof(int8_t), cudaMemcpyDeviceToHost, C));
-            }
-            rows_copied = rows_upto;
-            const int64_t n_new = (int64_t)(upto - copied);
-            if (n_new > 0 && copy_cloud) {
-                CU(cudaMemcpyAsync(sim->cloud_host.p + copied * 3, sim->cloud_dev.p + copied * 3,
-                                   (size_t)n_new * 3 * sizeof(double), cudaMemcpyDeviceToHost, C));
-                CU(cudaMemcpyAsync(sim->labels_host.p + copied, sim->labels_dev.p + copied,
-                                   (size_t)n_new * sizeof(int64_t), cudaMemcpyDeviceToHost, C));
-            }
-            if (n_new > 0 && use_columns) {
-                CU(cudaMemcpyAsync(sim->col_pad_host.p + copied, sim->col_pad_dev.p + copied,
-                                   (size_t)n_new * sizeof(int16_t), cudaMemcpyDeviceToHost, C));
-                if (use_packed)
-                    CU(cudaMemcpyAsync(sim->col_wig_host.p + copied, sim->col_wig_dev.p + copied,
-                                       (size_t)n_new * sizeof(uint16_t), cudaMemcpyDeviceToHost, C));
-                else
-                    CU(cudaMemcpyAsync(sim->col_tbq_host.p + copied, sim->col_tbq_dev.p + copied,
-                                       (size_t)n_new * sizeof(uint32_t), cudaMemcpyDeviceToHost, C));
-                if (use_q32)
-                    CU(cudaMemcpyAsync(sim->col_q32_host.p + copied, sim->col_q32_dev.p + copied,
-                                       (size_t)n_new * sizeof(uint32_t), cudaMemcpyDeviceToHost, C));
-                else
-                    CU(cudaMemcpyAsync(sim->col_q_host.p + copied, sim->col_q_dev.p + copied,
-                                       (size_t)n_new * sizeof(int64_t), cudaMemcpyDeviceToHost, C));
-                if (!use_packed)
-                    CU(cudaMemcpyAsync(sim->col_label_host.p + copied, sim->col_label_dev.p + copied,
-                                       (size_t)n_new * sizeof(int8_t), cudaMemcpyDeviceToHost, C));
-            }
+            const int r = copy_outputs(sim, op, b0, copied, upto);
+            if (r) return r;
             copy_marks.push_back({c0, sim->mark(C)});
             copied = upto;
-            copied_events = upto_event;
             return ATTPC_OK;
         };
         for (const ChunkFence& cf : fences) {
             CU(cudaEventSynchronize(cf.done));
             const unsigned long long upto = sim->chunk_totals.p[2 * cf.slot];
-            if ((int64_t)upto > sim->labels_dev.n) break;  // output overflow: the launch will be redone below
+            if ((int64_t)upto > sim->out_rows) break;  // output overflow: the launch will be redone below
             CU(cudaStreamWaitEvent(C, cf.done, 0));
-            rc = copy_rows(upto, sim->chunk_totals.p[2 * cf.slot + 1], cf.last_event);
+            rc = copy_rows(CopyMark{cf.last_event, upto, sim->chunk_totals.p[2 * cf.slot + 1]});
             if (rc) return rc;
         }
         CU(cudaEventSynchronize(groups_done));
@@ -962,60 +1065,7 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
             fin_marks.resize(fin_before);
             copy_marks.resize(copy_before);
             if (++retries > 24) return sim->fail(ATTPC_E_CAPACITY, "buffers still too small after 24 retries");
-            CU(cudaStreamSynchronize(T));  // the next launch's track kernel may be using buffers we are about to free
-            CU(cudaStreamSynchronize(C));
-            if (now.overflow_sub) {  // (overflow_points is raised with it: the point lists themselves were complete)
-                if (sim->sub_cap >= (1LL << 30)) return sim->fail(ATTPC_E_CAPACITY, "a group needs > 2^30 sub-points");
-                sim->sub_cap *= 2;
-                sim->geom.release(); sim->rec.release();
-                sim->unit_event.release(); sim->unit_first.release(); sim->unit_count.release();
-                sim->unit_order.release();
-            } else if (now.overflow_points) {
-                sim->group_point_cap *= 2;
-                for (auto& s2 : sim->slot) s2.release_points();
-                sim->geom.release(); sim->rec.release();
-                sim->unit_event.release(); sim->unit_first.release(); sim->unit_count.release();
-                sim->unit_order.release();
-            }
-            if (now.overflow_hash) {
-                if (sim->hash_cap >= (1 << 20)) return sim->fail(ATTPC_E_CAPACITY, "event needs > 2^20 hash slots");
-                sim->hash_cap *= 2;
-                sim->hash.release();
-                sim->sort_items.release();
-                sim->staged.release();
-            }
-            if (now.overflow_out) {
-                out_cap = std::max<int64_t>(sim->labels_dev.n * 2, (int64_t)sim->csr_host.p[0] + (1 << 20));
-                rc = ensure_out_buffers(sim, n_events, out_cap, true);
-                if (rc) return rc;
-                if (copy_cloud) {
-                    CU(sim->cloud_host.reserve(sim->cloud_dev.n, true));
-                    CU(sim->labels_host.reserve(sim->labels_dev.n, true));
-                }
-                if (use_columns) {
-                    CU(sim->col_pad_host.reserve(sim->labels_dev.n, true));
-                    CU(sim->col_tbq_host.reserve(sim->labels_dev.n, true));
-                    if (use_q32) CU(sim->col_q32_host.reserve(sim->labels_dev.n, true));
-                    else CU(sim->col_q_host.reserve(sim->labels_dev.n, true));
-                    CU(sim->col_label_host.reserve(sim->labels_dev.n, true));
-                    if (use_packed) CU(sim->col_wig_host.reserve(sim->labels_dev.n, true));
-                }
-                if (spy) {  // the row buffers follow the cloud buffers (device side: rows of finished launches are kept)
-                    if (spy_rows) {
-                        CU(sim->rows_dev.reserve(sim->labels_dev.n * 8, true, sim->stream));
-                        CU(sim->row_labels_dev.reserve(sim->labels_dev.n, true, sim->stream));
-                    } else {
-                        CU(sim->rcol_pad_dev.reserve(sim->labels_dev.n, true, sim->stream));
-                        CU(sim->rcol_tbq_dev.reserve(sim->labels_dev.n, true, sim->stream));
-                        CU(sim->rcol_elo_dev.reserve(sim->labels_dev.n, true, sim->stream));
-                        CU(sim->rcol_ehi_dev.reserve(sim->labels_dev.n, true, sim->stream));
-                        CU(sim->rcol_label_dev.reserve(sim->labels_dev.n, true, sim->stream));
-                    }
-                    rc = reserve_spyral(true);
-                    if (rc) return rc;
-                }
-            }
-            rc = ensure_work_buffers(sim, std::min<int64_t>(n_events, launch_cap), ranks, table_groups);
+            rc = grow_buffers(sim, now, op, n_events, work_events, ranks, table_groups);
             if (rc) return rc;
             sim->csr_host.p[0] = csr_before;  // forget the rows (and the big-count exceptions) of the failed attempt
             sim->csr_host.p[1] = big_before;
@@ -1026,106 +1076,28 @@ int run_batch(AttpcSim* sim, const LaunchPlan& plan, int64_t n_events, uint32_t 
             next_track = i;  // redo this launch (and the one that was running ahead)
             continue;
         }
-        totals.traj_points += now.traj_points;
-        totals.active_points += now.active_points;
-        totals.primary_electrons += now.primary_electrons;
-        totals.deposits += now.deposits;
-        totals.keys += now.keys;
-        totals.probes += now.probes;
-        totals.flushes += now.flushes;
-        totals.rk_steps += now.rk_steps;
-        totals.rk_rejects += now.rk_rejects;
-        totals.max_track_passes = std::max(totals.max_track_passes, now.max_track_passes);
+        add_counters(totals, now);
         const unsigned long long csr_after = sim->csr_host.p[0], rows_after = sim->csr_host.p[2];
         big_before = sim->csr_host.p[1];
-        if (copy_host && (copied < csr_after || rows_copied < rows_after || copied_events < nb)) {  // whatever the chunk copies did not cover
+        if (op.copy_host && (copied.cloud < csr_after || copied.spyral < rows_after || copied.events < nb)) {  // whatever the chunk copies did not cover
             CU(cudaStreamWaitEvent(C, groups_done, 0));
-            rc = copy_rows(csr_after, rows_after, nb);
+            rc = copy_rows(CopyMark{nb, csr_after, rows_after});
             if (rc) return rc;
         }
         csr_before = csr_after;
         rows_before = rows_after;
         ++i;
     }
-    const int64_t n_points = (int64_t)csr_before;
-    res->n_points = n_points;
-    res->offsets_dev = sim->offsets_dev.p;
-    if (want_cloud) {
-        res->cloud_dev = sim->cloud_dev.p;
-        res->labels_dev = sim->labels_dev.p;
+    if (op.use_q32 && (int64_t)big_before > sim->big_cap) {
+        // too many exceptions for the list (heavy ions): the full-width column, now and from now on
+        sim->q32_off = true;
+        CU(cudaStreamSynchronize(T));
+        CU(cudaStreamSynchronize(C));
+        CU(cudaStreamSynchronize(G));
+        return run_batch(sim, plan, n_events, flags, res, ms_h2d);
     }
-    res->n_trajectory_points = (int64_t)totals.traj_points;
-    res->n_active_points = (int64_t)totals.active_points;
-    res->n_primary_electrons = (int64_t)totals.primary_electrons;
-    res->n_deposits = (int64_t)totals.deposits;
-    res->n_keys = (int64_t)totals.keys;
-    res->n_hash_probes = (int64_t)totals.probes;
-    res->n_table_flushes = (int64_t)totals.flushes;
-    res->n_rk_steps = (int64_t)totals.rk_steps;
-    res->n_rk_rejects = (int64_t)totals.rk_rejects;
-    res->max_track_passes = (int64_t)totals.max_track_passes;
-    res->n_retries = retries;
-    if (copy_host) {
-        if (n_events == 0) {
-            CU(cudaMemcpyAsync(sim->offsets_host.p, sim->offsets_dev.p, sizeof(int64_t), cudaMemcpyDeviceToHost, C));
-        }
-        res->offsets = sim->offsets_host.p;
-        if (copy_cloud) {
-            res->cloud = sim->cloud_host.p;
-            res->labels = sim->labels_host.p;
-        }
-        if (use_columns) {
-            res->col_pad = sim->col_pad_host.p;
-            if (use_packed) {
-                res->col_wiggle = sim->col_wig_host.p;
-                res->tb_counts = sim->tbc_host.p;
-                res->pad_rank_shift = 14;
-            } else {
-                res->col_tb_q16 = sim->col_tbq_host.p;
-            }
-            if (!use_q32) {
-                res->col_electrons = sim->col_q_host.p;
-            } else if ((int64_t)big_before <= sim->big_cap) {
-                res->col_electrons32 = sim->col_q32_host.p;
-                res->n_big = (int64_t)big_before;
-                if (big_before > 0) {
-                    CU(sim->big_rows_host.reserve((int64_t)big_before));
-                    CU(sim->big_q_host.reserve((int64_t)big_before));
-                    CU(cudaMemcpyAsync(sim->big_rows_host.p, sim->big_rows_dev.p, (size_t)big_before * sizeof(int64_t),
-                                       cudaMemcpyDeviceToHost, C));
-                    CU(cudaMemcpyAsync(sim->big_q_host.p, sim->big_q_dev.p, (size_t)big_before * sizeof(int64_t),
-                                       cudaMemcpyDeviceToHost, C));
-                    res->big_rows = sim->big_rows_host.p;
-                    res->big_electrons = sim->big_q_host.p;
-                }
-            } else {  // too many exceptions for the list (heavy ions): the full-width column, now and from now on
-                sim->q32_off = true;
-                CU(cudaStreamSynchronize(T));
-                CU(cudaStreamSynchronize(C));
-                CU(cudaStreamSynchronize(G));
-                return run_batch(sim, plan, n_events, flags, res, ms_h2d);
-            }
-            if (!use_packed) res->col_label = sim->col_label_host.p;
-        }
-    }
-    if (spy) {
-        res->n_rows = (int64_t)rows_before;
-        if (copy_host) {
-            if (n_events == 0)
-                CU(cudaMemcpyAsync(sim->row_offsets_host.p, sim->row_offsets_dev.p, sizeof(int64_t), cudaMemcpyDeviceToHost, C));
-            res->row_offsets = sim->row_offsets_host.p;
-            if (spy_rows) {
-                res->rows = sim->rows_host.p;
-                res->row_labels = sim->row_labels_host.p;
-            } else {
-                res->row_col_pad = sim->rcol_pad_host.p;
-                res->row_col_tb_q16 = sim->rcol_tbq_host.p;
-                res->row_col_e_lo = sim->rcol_elo_host.p;
-                res->row_col_e_hi = sim->rcol_ehi_host.p;
-                res->row_col_label = sim->rcol_label_host.p;
-            }
-        }
-    }
+    rc = publish_result(sim, op, totals, retries, CopyMark{n_events, csr_before, rows_before}, big_before, res);
+    if (rc) return rc;
     // close the timeline on G after the other two streams have drained
     CU(cudaStreamWaitEvent(G, sim->fence(T), 0));
     CU(cudaStreamWaitEvent(G, sim->fence(C), 0));
@@ -1160,6 +1132,191 @@ int check_tracks(AttpcSim* sim, int32_t n_nuclei, const int32_t* track_nucleus, 
     return ATTPC_OK;
 }
 
+// attpc_create after its argument checks: streams, constants and tables of a new simulator on the current device.
+int init_sim(AttpcSim* sim, const AttpcConfig* cfg, const int16_t* pad_lut, const double* pad_xy, const double* pad_scale,
+             int32_t n_pads, const double* response, int32_t n_response, const AttpcSpecies* species, int32_t n_species) {
+    CU(cudaStreamCreateWithFlags(&sim->stream, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&sim->stream_t, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&sim->stream_c, cudaStreamNonBlocking));
+    int sm = 0;
+    CU(cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, sim->device));
+    sim->sm_count = sm > 0 ? sm : 148;
+
+    SimParams& P = sim->P;
+    P.length = cfg->length;
+    P.dv = cfg->drift_velocity;
+    P.mm_edge = (double)cfg->micromegas_edge;
+    P.win_edge = (double)cfg->windows_edge;
+    P.diffusion = cfg->diffusion;
+    P.long_diffusion = cfg->longitudinal_diffusion;
+    if (P.long_diffusion > 0.0) {  // widest window: sigma_L one bucket past the window edge (no point drifts longer)
+        const double t = P.win_edge + 1.0;
+        const double sl = std::sqrt(2.0 * P.long_diffusion * P.dv * t / cfg->efield) / P.dv;
+        if (!(sl < 1.0e6))
+            return sim->fail(ATTPC_E_BADARG, "attpc_create: longitudinal diffusion needs efield > 0 (sigma_L = %g)", sl);
+        sim->long_buckets = (int32_t)std::floor(6.0 * sl) + 2;
+    }
+    P.efield = cfg->efield;
+    P.fano = cfg->fano_factor;
+    P.ev_per_w = 1.0e6 / cfg->w_value;
+    P.B = cfg->bfield * -1.0;
+    P.E = cfg->efield * -1.0;
+    P.gain = cfg->mpgd_gain;
+    P.grid_low = cfg->grid_low_mm;
+    P.grid_high = cfg->grid_high_mm;
+    P.lut_origin = cfg->lut_origin_mm;
+    P.lut_n = cfg->lut_n;
+    P.adc_threshold = cfg->adc_threshold;
+    P.rtol = cfg->ode_rtol > 0 ? cfg->ode_rtol : 1e-6;
+    P.atol = cfg->ode_atol > 0 ? cfg->ode_atol : 1e-10;
+    P.freeze_ke = cfg->freeze_ke_mev;
+    P.lm = n_species ? species[0].lm : 0;
+    P.e_min = n_species ? species[0].e_min : 0;
+    P.n_oct = n_species ? species[0].n_oct : 0;
+    P.n_nodes = P.n_oct * (1 << P.lm) + 1;
+    P.n_species = n_species;
+    P.n_pads = n_pads;
+    P.n_response = n_response;
+    if (cfg->max_events_per_launch > 0) sim->launch_events = cfg->max_events_per_launch;
+    if (cfg->copy_events_per_launch > 0) sim->copy_launch_events = cfg->copy_events_per_launch;  // events per launch when rows go to the host
+    if (cfg->hash_capacity > 0) sim->hash_cap = next_pow2(cfg->hash_capacity);
+    if (cfg->unit_points > 0) sim->unit_points = std::min<int32_t>(cfg->unit_points, UNIT_POINTS);
+    if (cfg->table_spill_keys > 0) sim->spill_keys = std::min<int32_t>(cfg->table_spill_keys, SMEM_SPILL_AT);
+    sim->group_events = std::min(sim->group_events, sim->launch_events);
+    if (const char* env = getenv("ATTPC_CHUNK_GROUPS")) sim->chunk_groups = std::max(1, atoi(env));  // tuning aid
+    if (const char* env = getenv("ATTPC_BIG_CAP")) sim->big_cap = std::min<int64_t>(ATTPC_BIG_CAP, std::max(0, atoi(env)));  // tests
+
+    const int64_t lut_cells = (int64_t)cfg->lut_n * cfg->lut_n;
+    CU(sim->lut.reserve(lut_cells));
+    CU(cudaMemcpy(sim->lut.p, pad_lut, (size_t)lut_cells * sizeof(int16_t), cudaMemcpyHostToDevice));
+    CU(sim->pad_xy.reserve((int64_t)n_pads * 2));
+    CU(cudaMemcpy(sim->pad_xy.p, pad_xy, (size_t)n_pads * 2 * sizeof(double), cudaMemcpyHostToDevice));
+    CU(sim->pad_scale.reserve(n_pads));
+    CU(cudaMemcpy(sim->pad_scale.p, pad_scale, (size_t)n_pads * sizeof(double), cudaMemcpyHostToDevice));
+    CU(sim->response.reserve(n_response));
+    CU(cudaMemcpy(sim->response.p, response, (size_t)n_response * sizeof(double), cudaMemcpyHostToDevice));
+    {
+        std::vector<double> sorted(response, response + n_response);
+        std::sort(sorted.begin(), sorted.end(), [](double a, double b) { return a > b; });
+        std::vector<double> prefix(n_response + 1, 0.0);
+        for (int i = 0; i < n_response; ++i) prefix[i + 1] = prefix[i] + sorted[i];
+        CU(sim->resp_sorted.reserve(n_response));
+        CU(cudaMemcpy(sim->resp_sorted.p, sorted.data(), (size_t)n_response * sizeof(double), cudaMemcpyHostToDevice));
+        CU(sim->resp_prefix.reserve(n_response + 1));
+        CU(cudaMemcpy(sim->resp_prefix.p, prefix.data(), (size_t)(n_response + 1) * sizeof(double),
+                       cudaMemcpyHostToDevice));
+        P.resp_max = sorted[0];
+        // smallest electron count that passes the ADC threshold (detector/writer.py:232): amp = min(r_max e, 4095) is
+        // monotone in e, so the comparison can be made on the integer charge
+        {
+            const double thr = cfg->adc_threshold;
+            long long keep = 0;
+            if (!(thr < 4095.0)) {
+                keep = INT64_MAX;
+            } else if (thr >= 0.0 && sorted[0] > 0.0) {
+                keep = std::max<long long>(0, (long long)std::floor(thr / sorted[0]) - 2);
+                while (!(std::fmin(sorted[0] * (double)keep, 4095.0) > thr)) ++keep;
+            } else if (thr >= 0.0) {
+                keep = INT64_MAX;  // a null response never passes a non-negative threshold
+            }
+            P.e_keep_min = keep;
+        }
+    }
+    {
+        // deceleration tables: dE/dx [MeV/(g/cm^2)] * MEV_2_JOULE * density * 100 / m_kg / c  (detector/solver.py:64-76)
+        std::vector<double> scaled((size_t)n_species * P.n_nodes);
+        for (int s = 0; s < n_species; ++s) {
+            if (!species[s].dedx || !(species[s].mass > 0.0))
+                return sim->fail(ATTPC_E_BADARG, "species %d: null table or non-positive mass", s);
+            const double mass_kg = species[s].mass * MEV_2_KG;
+            const double scale = MEV_2_JOULE * cfg->gas_density * 100.0 / mass_kg / C_LIGHT;
+            for (int i = 0; i < P.n_nodes; ++i) scaled[(size_t)s * P.n_nodes + i] = species[s].dedx[i] * scale;
+            P.sp[s].mass = species[s].mass;
+            P.sp[s].qm_c = (double)species[s].z * E_CHARGE / mass_kg / C_LIGHT;
+            P.sp[s].z = species[s].z;
+            P.sp[s].table = s * P.n_nodes;
+            // terminal drift energy: first table node where the drag reaches the field acceleration |q E / (m c)|
+            {
+                const double field = std::fabs(P.sp[s].qm_c * P.E);
+                const double* t = &scaled[(size_t)s * P.n_nodes];
+                const int per_oct = 1 << P.lm;
+                double ke_eq = 0.0;
+                if (field > 0.0) {
+                    const double ke0 = std::ldexp(1.0, P.e_min);
+                    if (t[0] >= field) {  // below the table: drag = t[0] sqrt(ke / ke0)
+                        ke_eq = t[0] > 0.0 ? ke0 * (field / t[0]) * (field / t[0]) : 0.0;
+                    } else {
+                        for (int i = 1; i < P.n_nodes; ++i) {
+                            if (t[i] >= field) {
+                                auto node = [&](int j) {
+                                    return std::ldexp(1.0 + (double)(j % per_oct) / per_oct, P.e_min + j / per_oct);
+                                };
+                                const double f = (field - t[i - 1]) / (t[i] - t[i - 1]);
+                                ke_eq = node(i - 1) + f * (node(i) - node(i - 1));
+                                break;
+                            }
+                        }
+                    }
+                }
+                P.sp[s].ke_eq = ke_eq;
+            }
+        }
+        CU(sim->tables.reserve(std::max<int64_t>(1, (int64_t)scaled.size())));
+        if (!scaled.empty())
+            CU(cudaMemcpy(sim->tables.p, scaled.data(), scaled.size() * sizeof(double), cudaMemcpyHostToDevice));
+        // time [ns] to slow down from node i to node 0: integral of d(gamma beta) / deceleration (trapezoids); only the
+        // launch order of the tracks depends on it
+        std::vector<double> stop((size_t)n_species * P.n_nodes, 0.0);
+        for (int s = 0; s < n_species; ++s) {
+            const int per_oct = 1 << P.lm;
+            auto node = [&](int j) { return std::ldexp(1.0 + (double)(j % per_oct) / per_oct, P.e_min + j / per_oct); };
+            auto gb = [&](double ke) { const double g = ke / species[s].mass + 1.0; return std::sqrt(g * g - 1.0); };
+            const double* a = &scaled[(size_t)s * P.n_nodes];
+            double* out = &stop[(size_t)s * P.n_nodes];
+            for (int i = 1; i < P.n_nodes; ++i) {
+                const double mean = 0.5 * (a[i] + a[i - 1]);
+                out[i] = out[i - 1] + (mean > 0.0 ? (gb(node(i)) - gb(node(i - 1))) / mean * 1e9 : 0.0);
+            }
+        }
+        CU(sim->stop_ns.reserve(std::max<int64_t>(1, (int64_t)stop.size())));
+        if (!stop.empty())
+            CU(cudaMemcpy(sim->stop_ns.p, stop.data(), stop.size() * sizeof(double), cudaMemcpyHostToDevice));
+        sim->table_smem_bytes = scaled.size() * sizeof(double);
+        // the tables share the SM's 227 KB with the step slots of the warps: many species -> fewer warps per CTA;
+        // below four warps the tables stay in global memory (L1/L2) instead
+        const int64_t room = 227 * 1024 - (int64_t)sim->table_smem_bytes;
+        const int fit = (int)std::min<int64_t>(TRACK_THREADS / 32, room / (int64_t)TRACK_SLOT_BYTES_PER_WARP);
+        sim->tables_in_smem = fit >= 4;
+        sim->track_warps_max = sim->tables_in_smem ? fit : TRACK_THREADS / 32;
+    }
+    {
+        // constant mesh weights pdf * step^2 of detector/transporter.py:217-246 in exact arithmetic (sigma cancels):
+        // (36 / 81) / (2 pi) * exp(-(a_i^2 + a_j^2) / 2), a_i = -3 + 6 i / 9, rounded once from extended precision
+        const long double pi_l = 3.14159265358979323846264338327950288L;
+        for (int i = 0; i < MESH_N; ++i)
+            for (int j = 0; j < MESH_N; ++j) {
+                const long double ai = -3.0L + 6.0L * i / 9.0L, aj = -3.0L + 6.0L * j / 9.0L;
+                P.mesh_w[i * MESH_N + j] = (double)((2.0L / (9.0L * pi_l)) * expl(-(ai * ai + aj * aj) / 2.0L));
+            }
+        // the distinct values of the table (the mesh is symmetric): what the per-point exactness test multiplies
+        P.n_mesh_w_unique = 0;
+        for (int k = 0; k < MESH_N * MESH_N; ++k) {
+            bool seen = false;
+            for (int u = 0; u < P.n_mesh_w_unique; ++u) seen = seen || P.mesh_w_unique[u] == P.mesh_w[k];
+            if (!seen) P.mesh_w_unique[P.n_mesh_w_unique++] = P.mesh_w[k];
+        }
+    }
+    P.lut = sim->lut.p;
+    P.tables = sim->tables.p;
+    P.stop_ns = sim->stop_ns.p;
+    P.pad_xy = sim->pad_xy.p;
+    P.pad_scale = sim->pad_scale.p;
+    P.response = sim->response.p;
+    P.resp_sorted = sim->resp_sorted.p;
+    P.resp_prefix = sim->resp_prefix.p;
+    return ATTPC_OK;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------------------------------- C ABI
@@ -1178,36 +1335,6 @@ const char* attpc_last_error(const AttpcSim* sim) { return sim ? sim->error.c_st
 void attpc_destroy(AttpcSim* sim) {
     if (!sim) return;
     cudaSetDevice(sim->device);
-    if (sim->stream) cudaStreamSynchronize(sim->stream);
-    if (sim->stream_t) cudaStreamSynchronize(sim->stream_t);
-    if (sim->stream_c) cudaStreamSynchronize(sim->stream_c);
-    for (auto e : sim->events) cudaEventDestroy(e);
-    for (auto e : sim->sync_events) cudaEventDestroy(e);
-    for (auto& ls : sim->slot) ls.release_all();
-    sim->csr_total.release(); sim->csr_host.release(); sim->chunk_totals.release();
-    if (sim->stream_t) cudaStreamDestroy(sim->stream_t);
-    if (sim->stream_c) cudaStreamDestroy(sim->stream_c);
-    sim->lut.release(); sim->pad_xy.release(); sim->pad_scale.release(); sim->response.release();
-    sim->resp_sorted.release(); sim->resp_prefix.release(); sim->tables.release(); sim->stop_ns.release(); sim->plan_cls.release(); sim->plan_counts.release(); sim->plan_order.release();
-    sim->hash.release(); sim->sort_items.release(); sim->staged.release(); sim->big_list.release();
-    sim->geom.release(); sim->rec.release();
-    sim->nsub.release(); sim->sub_cnt.release(); sim->sub_start.release(); sim->sub_total.release();
-    sim->unit_event.release(); sim->unit_first.release(); sim->unit_count.release(); sim->unit_order.release();
-    sim->n_units.release();
-    sim->pstart.release(); sim->n_entries.release(); sim->mode.release();
-    sim->kept.release(); sim->in_momenta.release(); sim->in_vertices.release();
-    sim->offsets_dev.release(); sim->labels_dev.release(); sim->row_offsets_dev.release();
-    sim->row_labels_dev.release(); sim->cloud_dev.release(); sim->rows_dev.release(); sim->row_kept.release();
-    sim->row_sort_keys.release(); sim->row_sort_idx.release();
-    sim->rcol_pad_dev.release(); sim->rcol_tbq_dev.release(); sim->rcol_elo_dev.release(); sim->rcol_ehi_dev.release();
-    sim->rcol_label_dev.release(); sim->rcol_pad_host.release(); sim->rcol_tbq_host.release(); sim->rcol_elo_host.release();
-    sim->rcol_ehi_host.release(); sim->rcol_label_host.release();
-    sim->col_pad_dev.release(); sim->col_tbq_dev.release(); sim->col_q_dev.release(); sim->col_q32_dev.release(); sim->big_rows_dev.release(); sim->big_q_dev.release(); sim->col_label_dev.release();
-    sim->col_wig_dev.release(); sim->tbc_dev.release(); sim->col_wig_host.release(); sim->tbc_host.release();
-    sim->col_pad_host.release(); sim->col_tbq_host.release(); sim->col_q_host.release(); sim->col_q32_host.release(); sim->big_rows_host.release(); sim->big_q_host.release(); sim->col_label_host.release();
-    sim->offsets_host.release(); sim->labels_host.release(); sim->row_offsets_host.release();
-    sim->row_labels_host.release(); sim->cloud_host.release(); sim->rows_host.release();
-    if (sim->stream) cudaStreamDestroy(sim->stream);
     delete sim;
 }
 
@@ -1244,203 +1371,12 @@ int attpc_create(const AttpcConfig* cfg, const int16_t* pad_lut, const double* p
     AttpcSim* sim = new AttpcSim();
     sim->device = device;
     sim->cfg = *cfg;
-    auto bail = [&](int code) {
+    const int rc = init_sim(sim, cfg, pad_lut, pad_xy, pad_scale, n_pads, response, n_response, species, n_species);
+    if (rc) {
         g_create_error = sim->error;
-        attpc_destroy(sim);
-        return code;
-    };
-#define CUC(call)                                                                                   \
-    do {                                                                                            \
-        cudaError_t _e = (call);                                                                    \
-        if (_e != cudaSuccess) {                                                                    \
-            sim->fail(ATTPC_E_CUDA, "%s failed: %s", #call, cudaGetErrorString(_e));                \
-            return bail(ATTPC_E_CUDA);                                                              \
-        }                                                                                           \
-    } while (0)
-    CUC(cudaStreamCreateWithFlags(&sim->stream, cudaStreamNonBlocking));
-    CUC(cudaStreamCreateWithFlags(&sim->stream_t, cudaStreamNonBlocking));
-    CUC(cudaStreamCreateWithFlags(&sim->stream_c, cudaStreamNonBlocking));
-    int sm = 0;
-    CUC(cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, device));
-    sim->sm_count = sm > 0 ? sm : 148;
-
-    SimParams& P = sim->P;
-    P.length = cfg->length;
-    P.dv = cfg->drift_velocity;
-    P.mm_edge = (double)cfg->micromegas_edge;
-    P.win_edge = (double)cfg->windows_edge;
-    P.diffusion = cfg->diffusion;
-    P.long_diffusion = cfg->longitudinal_diffusion;
-    if (P.long_diffusion > 0.0) {  // widest window: sigma_L one bucket past the window edge (no point drifts longer)
-        const double t = P.win_edge + 1.0;
-        const double sl = std::sqrt(2.0 * P.long_diffusion * P.dv * t / cfg->efield) / P.dv;
-        if (!(sl < 1.0e6)) {
-            sim->fail(ATTPC_E_BADARG, "attpc_create: longitudinal diffusion needs efield > 0 (sigma_L = %g)", sl);
-            return bail(ATTPC_E_BADARG);
-        }
-        sim->long_buckets = (int32_t)std::floor(6.0 * sl) + 2;
+        delete sim;
+        return rc;
     }
-    P.efield = cfg->efield;
-    P.fano = cfg->fano_factor;
-    P.ev_per_w = 1.0e6 / cfg->w_value;
-    P.B = cfg->bfield * -1.0;
-    P.E = cfg->efield * -1.0;
-    P.gain = cfg->mpgd_gain;
-    P.grid_low = cfg->grid_low_mm;
-    P.grid_high = cfg->grid_high_mm;
-    P.lut_origin = cfg->lut_origin_mm;
-    P.lut_n = cfg->lut_n;
-    P.adc_threshold = cfg->adc_threshold;
-    P.rtol = cfg->ode_rtol > 0 ? cfg->ode_rtol : 1e-6;
-    P.atol = cfg->ode_atol > 0 ? cfg->ode_atol : 1e-10;
-    P.freeze_ke = cfg->freeze_ke_mev;
-    P.lm = n_species ? species[0].lm : 0;
-    P.e_min = n_species ? species[0].e_min : 0;
-    P.n_oct = n_species ? species[0].n_oct : 0;
-    P.n_nodes = P.n_oct * (1 << P.lm) + 1;
-    P.n_species = n_species;
-    P.n_pads = n_pads;
-    P.n_response = n_response;
-    if (cfg->max_events_per_launch > 0) sim->launch_events = cfg->max_events_per_launch;
-    if (cfg->copy_events_per_launch > 0) sim->copy_launch_events = cfg->copy_events_per_launch;  // events per launch when rows go to the host
-    if (cfg->hash_capacity > 0) sim->hash_cap = next_pow2(cfg->hash_capacity);
-    if (cfg->unit_points > 0) sim->unit_points = std::min<int32_t>(cfg->unit_points, UNIT_POINTS);
-    if (cfg->table_spill_keys > 0) sim->spill_keys = std::min<int32_t>(cfg->table_spill_keys, SMEM_SPILL_AT);
-    sim->group_events = std::min(sim->group_events, sim->launch_events);
-    if (const char* env = getenv("ATTPC_CHUNK_GROUPS")) sim->chunk_groups = std::max(1, atoi(env));  // tuning aid
-    if (const char* env = getenv("ATTPC_BIG_CAP")) sim->big_cap = std::min<int64_t>(ATTPC_BIG_CAP, std::max(0, atoi(env)));  // tests
-
-    const int64_t lut_cells = (int64_t)cfg->lut_n * cfg->lut_n;
-    CUC(sim->lut.reserve(lut_cells));
-    CUC(cudaMemcpy(sim->lut.p, pad_lut, (size_t)lut_cells * sizeof(int16_t), cudaMemcpyHostToDevice));
-    CUC(sim->pad_xy.reserve((int64_t)n_pads * 2));
-    CUC(cudaMemcpy(sim->pad_xy.p, pad_xy, (size_t)n_pads * 2 * sizeof(double), cudaMemcpyHostToDevice));
-    CUC(sim->pad_scale.reserve(n_pads));
-    CUC(cudaMemcpy(sim->pad_scale.p, pad_scale, (size_t)n_pads * sizeof(double), cudaMemcpyHostToDevice));
-    CUC(sim->response.reserve(n_response));
-    CUC(cudaMemcpy(sim->response.p, response, (size_t)n_response * sizeof(double), cudaMemcpyHostToDevice));
-    {
-        std::vector<double> sorted(response, response + n_response);
-        std::sort(sorted.begin(), sorted.end(), [](double a, double b) { return a > b; });
-        std::vector<double> prefix(n_response + 1, 0.0);
-        for (int i = 0; i < n_response; ++i) prefix[i + 1] = prefix[i] + sorted[i];
-        CUC(sim->resp_sorted.reserve(n_response));
-        CUC(cudaMemcpy(sim->resp_sorted.p, sorted.data(), (size_t)n_response * sizeof(double), cudaMemcpyHostToDevice));
-        CUC(sim->resp_prefix.reserve(n_response + 1));
-        CUC(cudaMemcpy(sim->resp_prefix.p, prefix.data(), (size_t)(n_response + 1) * sizeof(double),
-                       cudaMemcpyHostToDevice));
-        P.resp_max = sorted[0];
-        // smallest electron count that passes the ADC threshold (detector/writer.py:232): amp = min(r_max e, 4095) is
-        // monotone in e, so the comparison can be made on the integer charge
-        {
-            const double thr = cfg->adc_threshold;
-            long long keep = 0;
-            if (!(thr < 4095.0)) {
-                keep = INT64_MAX;
-            } else if (thr >= 0.0 && sorted[0] > 0.0) {
-                keep = std::max<long long>(0, (long long)std::floor(thr / sorted[0]) - 2);
-                while (!(std::fmin(sorted[0] * (double)keep, 4095.0) > thr)) ++keep;
-            } else if (thr >= 0.0) {
-                keep = INT64_MAX;  // a null response never passes a non-negative threshold
-            }
-            P.e_keep_min = keep;
-        }
-    }
-    {
-        // deceleration tables: dE/dx [MeV/(g/cm^2)] * MEV_2_JOULE * density * 100 / m_kg / c  (detector/solver.py:64-76)
-        std::vector<double> scaled((size_t)n_species * P.n_nodes);
-        for (int s = 0; s < n_species; ++s) {
-            if (!species[s].dedx || !(species[s].mass > 0.0)) {
-                sim->fail(ATTPC_E_BADARG, "species %d: null table or non-positive mass", s);
-                return bail(ATTPC_E_BADARG);
-            }
-            const double mass_kg = species[s].mass * MEV_2_KG;
-            const double scale = MEV_2_JOULE * cfg->gas_density * 100.0 / mass_kg / C_LIGHT;
-            for (int i = 0; i < P.n_nodes; ++i) scaled[(size_t)s * P.n_nodes + i] = species[s].dedx[i] * scale;
-            P.sp[s].mass = species[s].mass;
-            P.sp[s].qm_c = (double)species[s].z * E_CHARGE / mass_kg / C_LIGHT;
-            P.sp[s].z = species[s].z;
-            P.sp[s].table = s * P.n_nodes;
-            // terminal drift energy: first table node where the drag reaches the field acceleration |q E / (m c)|
-            {
-                const double field = std::fabs(P.sp[s].qm_c * P.E);
-                const double* t = &scaled[(size_t)s * P.n_nodes];
-                const int per_oct = 1 << P.lm;
-                double ke_eq = 0.0;
-                if (field > 0.0) {
-                    const double ke0 = std::ldexp(1.0, P.e_min);
-                    if (t[0] >= field) {  // below the table: drag = t[0] sqrt(ke / ke0)
-                        ke_eq = t[0] > 0.0 ? ke0 * (field / t[0]) * (field / t[0]) : 0.0;
-                    } else {
-                        for (int i = 1; i < P.n_nodes; ++i) {
-                            if (t[i] >= field) {
-                                auto node = [&](int j) {
-                                    return std::ldexp(1.0 + (double)(j % per_oct) / per_oct, P.e_min + j / per_oct);
-                                };
-                                const double f = (field - t[i - 1]) / (t[i] - t[i - 1]);
-                                ke_eq = node(i - 1) + f * (node(i) - node(i - 1));
-                                break;
-                            }
-                        }
-                    }
-                }
-                P.sp[s].ke_eq = ke_eq;
-            }
-        }
-        CUC(sim->tables.reserve(std::max<int64_t>(1, (int64_t)scaled.size())));
-        if (!scaled.empty())
-            CUC(cudaMemcpy(sim->tables.p, scaled.data(), scaled.size() * sizeof(double), cudaMemcpyHostToDevice));
-        // time [ns] to slow down from node i to node 0: integral of d(gamma beta) / deceleration (trapezoids); only the
-        // launch order of the tracks depends on it
-        std::vector<double> stop((size_t)n_species * P.n_nodes, 0.0);
-        for (int s = 0; s < n_species; ++s) {
-            const int per_oct = 1 << P.lm;
-            auto node = [&](int j) { return std::ldexp(1.0 + (double)(j % per_oct) / per_oct, P.e_min + j / per_oct); };
-            auto gb = [&](double ke) { const double g = ke / species[s].mass + 1.0; return std::sqrt(g * g - 1.0); };
-            const double* a = &scaled[(size_t)s * P.n_nodes];
-            double* out = &stop[(size_t)s * P.n_nodes];
-            for (int i = 1; i < P.n_nodes; ++i) {
-                const double mean = 0.5 * (a[i] + a[i - 1]);
-                out[i] = out[i - 1] + (mean > 0.0 ? (gb(node(i)) - gb(node(i - 1))) / mean * 1e9 : 0.0);
-            }
-        }
-        CUC(sim->stop_ns.reserve(std::max<int64_t>(1, (int64_t)stop.size())));
-        if (!stop.empty())
-            CUC(cudaMemcpy(sim->stop_ns.p, stop.data(), stop.size() * sizeof(double), cudaMemcpyHostToDevice));
-        sim->table_smem_bytes = scaled.size() * sizeof(double);
-        // the tables share the SM's 227 KB with the step slots of the warps: many species -> fewer warps per CTA;
-        // below four warps the tables stay in global memory (L1/L2) instead
-        const int64_t room = 227 * 1024 - (int64_t)sim->table_smem_bytes;
-        const int fit = (int)std::min<int64_t>(TRACK_THREADS / 32, room / (int64_t)TRACK_SLOT_BYTES_PER_WARP);
-        sim->tables_in_smem = fit >= 4;
-        sim->track_warps_max = sim->tables_in_smem ? fit : TRACK_THREADS / 32;
-    }
-    {
-        // constant mesh weights pdf * step^2 of detector/transporter.py:217-246 in exact arithmetic (sigma cancels):
-        // (36 / 81) / (2 pi) * exp(-(a_i^2 + a_j^2) / 2), a_i = -3 + 6 i / 9, rounded once from extended precision
-        const long double pi_l = 3.14159265358979323846264338327950288L;
-        for (int i = 0; i < MESH_N; ++i)
-            for (int j = 0; j < MESH_N; ++j) {
-                const long double ai = -3.0L + 6.0L * i / 9.0L, aj = -3.0L + 6.0L * j / 9.0L;
-                P.mesh_w[i * MESH_N + j] = (double)((2.0L / (9.0L * pi_l)) * expl(-(ai * ai + aj * aj) / 2.0L));
-            }
-        // the distinct values of the table (the mesh is symmetric): what the per-point exactness test multiplies
-        P.n_mesh_w_unique = 0;
-        for (int k = 0; k < MESH_N * MESH_N; ++k) {
-            bool seen = false;
-            for (int u = 0; u < P.n_mesh_w_unique; ++u) seen = seen || P.mesh_w_unique[u] == P.mesh_w[k];
-            if (!seen) P.mesh_w_unique[P.n_mesh_w_unique++] = P.mesh_w[k];
-        }
-    }
-    P.lut = sim->lut.p;
-    P.tables = sim->tables.p;
-    P.stop_ns = sim->stop_ns.p;
-    P.pad_xy = sim->pad_xy.p;
-    P.pad_scale = sim->pad_scale.p;
-    P.response = sim->response.p;
-    P.resp_sorted = sim->resp_sorted.p;
-    P.resp_prefix = sim->resp_prefix.p;
-#undef CUC
     *out = sim;
     return ATTPC_OK;
 }
@@ -1531,37 +1467,25 @@ int attpc_simulate_replay(AttpcSim* sim, const int64_t* track_offsets, const dou
     DevArray<double> d_rows, d_norm, d_uvals;
     DevArray<int32_t> d_ev, d_rank, d_sp, d_lab;
     DevArray<long long> d_el;
-    auto cleanup = [&]() {
-        d_off.release(); d_ukeys.release(); d_uoff.release(); d_rows.release(); d_norm.release();
-        d_uvals.release(); d_ev.release(); d_rank.release(); d_sp.release(); d_lab.release(); d_el.release();
-    };
-#define CUR(call)                                                                                      \
-    do {                                                                                               \
-        cudaError_t _e = (call);                                                                       \
-        if (_e != cudaSuccess) {                                                                       \
-            cleanup();                                                                                 \
-            return sim->fail(ATTPC_E_CUDA, "%s failed: %s", #call, cudaGetErrorString(_e));            \
-        }                                                                                              \
-    } while (0)
     auto up = [&](auto& arr, const auto* src, int64_t n) -> cudaError_t {
         cudaError_t e = arr.reserve(std::max<int64_t>(1, n));
         if (e != cudaSuccess || n == 0) return e;
         return cudaMemcpyAsync(arr.p, src, (size_t)n * sizeof(*src), cudaMemcpyHostToDevice, sim->stream);
     };
-    CUR(up(d_off, track_offsets, n_tracks + 1));
-    CUR(up(d_rows, points, n_rows * 6));
-    CUR(up(d_norm, normals, n_rows));
-    CUR(up(d_ev, track_event, n_tracks));
-    CUR(up(d_rank, track_rank, n_tracks));
-    CUR(up(d_sp, track_species, n_tracks));
-    CUR(up(d_lab, label_map.data(), (int64_t)label_map.size()));
-    if (electrons_out) CUR(d_el.reserve(std::max<int64_t>(1, n_rows)));
+    CU(up(d_off, track_offsets, n_tracks + 1));
+    CU(up(d_rows, points, n_rows * 6));
+    CU(up(d_norm, normals, n_rows));
+    CU(up(d_ev, track_event, n_tracks));
+    CU(up(d_rank, track_rank, n_tracks));
+    CU(up(d_sp, track_species, n_tracks));
+    CU(up(d_lab, label_map.data(), (int64_t)label_map.size()));
+    if (electrons_out) CU(d_el.reserve(std::max<int64_t>(1, n_rows)));
     LaunchPlan plan;
     if (replay && replay->u_offsets) {
         const int64_t nu = replay->u_offsets[n_events];
-        CUR(up(d_uoff, replay->u_offsets, n_events + 1));
-        CUR(up(d_ukeys, replay->u_keys, nu));
-        CUR(up(d_uvals, replay->u_vals, nu));
+        CU(up(d_uoff, replay->u_offsets, n_events + 1));
+        CU(up(d_ukeys, replay->u_keys, nu));
+        CU(up(d_uvals, replay->u_vals, nu));
         plan.uniforms = ReplayUniforms{d_uoff.p, d_ukeys.p, d_uvals.p};
     }
     ReplayBatch rb;
@@ -1577,16 +1501,12 @@ int attpc_simulate_replay(AttpcSim* sim, const int64_t* track_offsets, const dou
     plan.replay = &rb;
     plan.label_of_event_rank_dev = d_lab.p;
     plan.n_tracks_per_event = t_max;
-    int rc = run_batch(sim, plan, n_events, flags, result, 0.f);
-    if (rc == ATTPC_OK && electrons_out && n_rows > 0) {
-        cudaError_t e = cudaMemcpy(electrons_out, d_el.p, (size_t)n_rows * sizeof(long long), cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) rc = sim->fail(ATTPC_E_CUDA, "electrons copy failed: %s", cudaGetErrorString(e));
-    }
-    if (rc == ATTPC_OK) result->n_tracks = n_tracks;
-    cudaStreamSynchronize(sim->stream);
-    cleanup();
-#undef CUR
-    return rc;
+    const int rc = run_batch(sim, plan, n_events, flags, result, 0.f);
+    if (rc) return rc;
+    if (electrons_out && n_rows > 0)
+        CU(cudaMemcpy(electrons_out, d_el.p, (size_t)n_rows * sizeof(long long), cudaMemcpyDeviceToHost));
+    result->n_tracks = n_tracks;
+    return ATTPC_OK;
 }
 
 int attpc_trajectories(AttpcSim* sim, const double* momenta, const double* vertices, const int32_t* species,
@@ -1603,21 +1523,17 @@ int attpc_trajectories(AttpcSim* sim, const double* momenta, const double* verti
     if (rc) return rc;
     DevArray<double> d_m, d_v, d_out;
     DevArray<int32_t> d_sp, d_cnt;
-    auto cleanup = [&]() { d_m.release(); d_v.release(); d_out.release(); d_sp.release(); d_cnt.release(); };
-    cudaError_t e = cudaSuccess;
-    auto ok = [&](cudaError_t x) { if (e == cudaSuccess) e = x; return e == cudaSuccess; };
-    ok(d_m.reserve(n_tracks * 4)) && ok(d_v.reserve(n_tracks * 3)) && ok(d_sp.reserve(n_tracks)) &&
-        ok(d_cnt.reserve(n_tracks)) && ok(d_out.reserve(n_tracks * max_points * 6)) &&
-        ok(cudaMemcpyAsync(d_m.p, momenta, (size_t)n_tracks * 4 * sizeof(double), cudaMemcpyHostToDevice, sim->stream)) &&
-        ok(cudaMemcpyAsync(d_v.p, vertices, (size_t)n_tracks * 3 * sizeof(double), cudaMemcpyHostToDevice, sim->stream)) &&
-        ok(cudaMemcpyAsync(d_sp.p, species, (size_t)n_tracks * sizeof(int32_t), cudaMemcpyHostToDevice, sim->stream)) &&
-        ok(cudaMemsetAsync(d_out.p, 0, (size_t)n_tracks * max_points * 6 * sizeof(double), sim->stream)) &&
-        ok(cudaMemsetAsync(d_cnt.p, 0, (size_t)n_tracks * sizeof(int32_t), sim->stream)) &&
-        ok(cudaMemsetAsync(sim->slot[0].counters.p, 0, sizeof(Counters), sim->stream));
-    if (e != cudaSuccess) {
-        cleanup();
-        return sim->fail(ATTPC_E_CUDA, "attpc_trajectories setup: %s", cudaGetErrorString(e));
-    }
+    CU(d_m.reserve(n_tracks * 4));
+    CU(d_v.reserve(n_tracks * 3));
+    CU(d_sp.reserve(n_tracks));
+    CU(d_cnt.reserve(n_tracks));
+    CU(d_out.reserve(n_tracks * max_points * 6));
+    CU(cudaMemcpyAsync(d_m.p, momenta, (size_t)n_tracks * 4 * sizeof(double), cudaMemcpyHostToDevice, sim->stream));
+    CU(cudaMemcpyAsync(d_v.p, vertices, (size_t)n_tracks * 3 * sizeof(double), cudaMemcpyHostToDevice, sim->stream));
+    CU(cudaMemcpyAsync(d_sp.p, species, (size_t)n_tracks * sizeof(int32_t), cudaMemcpyHostToDevice, sim->stream));
+    CU(cudaMemsetAsync(d_out.p, 0, (size_t)n_tracks * max_points * 6 * sizeof(double), sim->stream));
+    CU(cudaMemsetAsync(d_cnt.p, 0, (size_t)n_tracks * sizeof(int32_t), sim->stream));
+    CU(cudaMemsetAsync(sim->slot[0].counters.p, 0, sizeof(Counters), sim->stream));
     TrackBatch tb;
     memset(&tb, 0, sizeof tb);
     tb.momenta = d_m.p;
@@ -1631,16 +1547,12 @@ int attpc_trajectories(AttpcSim* sim, const double* momenta, const double* verti
     tb.rec_stride = stride;
     tb.rec_max = max_points;
     rc = launch_tracks<true>(sim, tb, n_tracks, 0, sim->stream);
-    if (rc == ATTPC_OK) {
-        ok(cudaMemcpyAsync(out_points, d_out.p, (size_t)n_tracks * max_points * 6 * sizeof(double),
-                           cudaMemcpyDeviceToHost, sim->stream)) &&
-            ok(cudaMemcpyAsync(out_counts, d_cnt.p, (size_t)n_tracks * sizeof(int32_t), cudaMemcpyDeviceToHost,
-                               sim->stream)) &&
-            ok(cudaStreamSynchronize(sim->stream));
-        if (e != cudaSuccess) rc = sim->fail(ATTPC_E_CUDA, "attpc_trajectories: %s", cudaGetErrorString(e));
-    }
-    cleanup();
-    return rc;
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(out_points, d_out.p, (size_t)n_tracks * max_points * 6 * sizeof(double), cudaMemcpyDeviceToHost,
+                       sim->stream));
+    CU(cudaMemcpyAsync(out_counts, d_cnt.p, (size_t)n_tracks * sizeof(int32_t), cudaMemcpyDeviceToHost, sim->stream));
+    CU(cudaStreamSynchronize(sim->stream));
+    return ATTPC_OK;
 }
 
 int attpc_convert_to_spyral(AttpcSim* sim, const int64_t* offsets, const double* cloud, const int64_t* labels,
@@ -1654,21 +1566,45 @@ int attpc_convert_to_spyral(AttpcSim* sim, const int64_t* offsets, const double*
     memset(result, 0, sizeof *result);
     sim->events_used = 0;
     sim->launches = 0;
-    int rc = ensure_out_buffers(sim, n_events, std::max<int64_t>(1, n_points), false);
+    OutputPlan op;  // the cloud comes from the host; the rows go back in one copy once they are counted
+    op.spy = op.spy_rows = true;
+    op.cloud_rows = {{&sim->cloud, false}, {&sim->labels, false}};
+    op.spyral_rows = {{&sim->rows, false}, {&sim->row_labels, false}};
+    int rc = reserve_outputs(sim, op, n_events, std::max<int64_t>(1, n_points), false);
     if (rc) return rc;
     CU(cudaMemcpyAsync(sim->offsets_dev.p, offsets, (size_t)(n_events + 1) * sizeof(int64_t), cudaMemcpyHostToDevice,
                        sim->stream));
     if (n_points > 0) {
-        CU(cudaMemcpyAsync(sim->cloud_dev.p, cloud, (size_t)n_points * 3 * sizeof(double), cudaMemcpyHostToDevice,
+        CU(cudaMemcpyAsync(sim->cloud.d(), cloud, (size_t)n_points * 3 * sizeof(double), cudaMemcpyHostToDevice,
                            sim->stream));
-        CU(cudaMemcpyAsync(sim->labels_dev.p, labels, (size_t)n_points * sizeof(int64_t), cudaMemcpyHostToDevice,
+        CU(cudaMemcpyAsync(sim->labels.d(), labels, (size_t)n_points * sizeof(int64_t), cudaMemcpyHostToDevice,
                            sim->stream));
     }
     result->n_events = n_events;
     result->n_points = n_points;
-    rc = run_spyral(sim, n_events, n_points, result, true, (flags & ATTPC_ROWS_KEEP_ALL) != 0);
+    CU(sim->csr_total.reserve(3));
+    CU(cudaMemsetAsync(sim->csr_total.p + 2, 0, sizeof(unsigned long long), sim->stream));
+    CU(cudaMemsetAsync(sim->row_offsets_dev.p, 0, sizeof(int64_t), sim->stream));
+    rc = launch_spyral(sim, spyral_args(sim, 0, n_events, false, (flags & ATTPC_ROWS_KEEP_ALL) != 0, nullptr));
+    if (rc) return rc;
+    CU(sim->row_offsets_host.reserve(n_events + 1));
+    CU(cudaMemcpyAsync(sim->row_offsets_host.p, sim->row_offsets_dev.p, (size_t)(n_events + 1) * sizeof(int64_t),
+                       cudaMemcpyDeviceToHost, sim->stream));
+    CU(cudaStreamSynchronize(sim->stream));
+    const int64_t n_rows = sim->row_offsets_host.p[n_events];
+    result->n_rows = n_rows;
+    result->row_offsets = sim->row_offsets_host.p;
+    CU(sim->rows.reserve_host(std::max<int64_t>(1, n_rows), false));
+    CU(sim->row_labels.reserve_host(std::max<int64_t>(1, n_rows), false));
+    if (n_rows > 0) {
+        CU(sim->rows.copy_to_host(0, n_rows, sim->stream));
+        CU(sim->row_labels.copy_to_host(0, n_rows, sim->stream));
+    }
+    CU(cudaStreamSynchronize(sim->stream));
+    result->rows = sim->rows.h();
+    result->row_labels = sim->row_labels.h();
     result->n_kernel_launches = sim->launches;
-    return rc;
+    return ATTPC_OK;
 }
 
 int attpc_read_device(AttpcSim* sim, const void* dev, void* host, int64_t n_bytes) {
@@ -1688,18 +1624,13 @@ int attpc_lookup_pads(AttpcSim* sim, const double* xy, int64_t n, int32_t* pads_
     CU(cudaSetDevice(sim->device));
     DevArray<double> d_xy;
     DevArray<int32_t> d_out;
-    cudaError_t e = d_xy.reserve(n * 2);
-    if (e == cudaSuccess) e = d_out.reserve(n);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_xy.p, xy, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, sim->stream);
-    if (e == cudaSuccess) {
-        lookup_kernel<<<(unsigned)((n + 255) / 256), 256, 0, sim->stream>>>(sim->P, d_xy.p, n, d_out.p);
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess) e = cudaMemcpyAsync(pads_out, d_out.p, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, sim->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(sim->stream);
-    d_xy.release();
-    d_out.release();
-    if (e != cudaSuccess) return sim->fail(ATTPC_E_CUDA, "attpc_lookup_pads: %s", cudaGetErrorString(e));
+    CU(d_xy.reserve(n * 2));
+    CU(d_out.reserve(n));
+    CU(cudaMemcpyAsync(d_xy.p, xy, (size_t)n * 2 * sizeof(double), cudaMemcpyHostToDevice, sim->stream));
+    lookup_kernel<<<(unsigned)((n + 255) / 256), 256, 0, sim->stream>>>(sim->P, d_xy.p, n, d_out.p);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(pads_out, d_out.p, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, sim->stream));
+    CU(cudaStreamSynchronize(sim->stream));
     return ATTPC_OK;
 }
 
