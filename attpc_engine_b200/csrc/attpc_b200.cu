@@ -185,6 +185,8 @@ struct AttpcSim {
     DevArray<unsigned> pstart, n_entries, mode;
     int32_t ranks = 1;
     int32_t max_units = 0;
+    int deposit_ctas = 0;                 // persistent deposit CTAs: as many as are resident at once
+    DevArray<unsigned> deposit_cursor;    // next work unit of the chunk, zeroed before every deposit launch
     // longitudinal diffusion (P.long_diffusion > 0): geom / rec then hold the SUB-POINTS (one per time bucket of a
     // point's window) of one chunk of at most SUB_CHUNK_GROUPS groups, sub_cap per group
     int64_t sub_cap = 0;
@@ -460,10 +462,10 @@ int run_groups(AttpcSim* sim, int64_t launch_events, FinalizeArgs fa, int which,
     auto far_kernel = order_queue_kernel<FIN_THREADS, 0, 2>;
     CU(cudaFuncSetAttribute(big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FIN_BIG_SMEM_BYTES));
     CU(cudaFuncSetAttribute(order_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FIN_SMEM_BYTES));
-    CU(cudaFuncSetAttribute(deposit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DEPOSIT_SMEM_BYTES));
-    // Groups are processed in chunks: every kernel is launched once per chunk with one grid row per group, so the
-    // ramp-up and tail of a launch are paid once per chunk.  When rows go to the host a chunk is what is copied while
-    // the next chunk computes; otherwise it is as many groups as the tables are sized for.
+    // Groups are processed in chunks: every kernel is launched once per chunk with one grid row per group (the deposit
+    // kernel's persistent CTAs walk the chunk's groups in turn), so the ramp-up and tail of a launch are paid once per
+    // chunk.  When rows go to the host a chunk is what is copied while the next chunk computes; otherwise it is as many
+    // groups as the tables are sized for.
     const bool split = sim->P.long_diffusion > 0.0;
     int64_t gpc = std::max<int64_t>(1, fences ? groups_per_chunk : sim->chunk_groups);
     if (split) gpc = std::min<int64_t>(gpc, SUB_CHUNK_GROUPS);
@@ -499,14 +501,15 @@ int run_groups(AttpcSim* sim, int64_t launch_events, FinalizeArgs fa, int which,
         }
         CU(cudaMemsetAsync(sim->n_entries.p + gv.first_slot, 0, (size_t)gv.n_events * sizeof(unsigned), sim->stream));
         cudaEvent_t k0 = sim->mark();
+        CU(cudaMemsetAsync(sim->deposit_cursor.p, 0, sizeof(unsigned), sim->stream));
         if (!split) {
-            deposit_kernel<<<dim3((unsigned)sim->max_units, (unsigned)ng), DEPOSIT_THREADS, DEPOSIT_SMEM_BYTES,
-                             sim->stream>>>(sim->P, pb, gv, ctr);
+            deposit_kernel<<<(unsigned)sim->deposit_ctas, DEPOSIT_THREADS, DEPOSIT_SMEM_BYTES, sim->stream>>>(
+                sim->P, pb, gv, (int)ng, sim->deposit_cursor.p, ctr);
         } else {
             GroupView gvs = gv;
             gvs.group = 0;
-            deposit_kernel<<<dim3((unsigned)sim->sub_max_units, (unsigned)ng), DEPOSIT_THREADS, DEPOSIT_SMEM_BYTES,
-                             sim->stream>>>(sim->P, sub_buf(sim, which, g0), gvs, ctr);
+            deposit_kernel<<<(unsigned)sim->deposit_ctas, DEPOSIT_THREADS, DEPOSIT_SMEM_BYTES, sim->stream>>>(
+                sim->P, sub_buf(sim, which, g0), gvs, (int)ng, sim->deposit_cursor.p, ctr);
         }
         cudaEvent_t d1 = sim->mark();
         CU(cudaMemsetAsync(qbase, 0, 4 * sizeof(unsigned), sim->stream));
@@ -1141,6 +1144,12 @@ int init_sim(AttpcSim* sim, const AttpcConfig* cfg, const int16_t* pad_lut, cons
     int sm = 0;
     CU(cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, sim->device));
     sim->sm_count = sm > 0 ? sm : 148;
+    CU(cudaFuncSetAttribute(deposit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DEPOSIT_SMEM_BYTES));
+    int deposit_per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&deposit_per_sm, deposit_kernel, DEPOSIT_THREADS,
+                                                     DEPOSIT_SMEM_BYTES));
+    sim->deposit_ctas = std::max(1, deposit_per_sm) * sim->sm_count;
+    CU(sim->deposit_cursor.reserve(1));
 
     SimParams& P = sim->P;
     P.length = cfg->length;

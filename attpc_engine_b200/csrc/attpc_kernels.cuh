@@ -11,9 +11,9 @@
 //                     columns of the 10x10 mesh of every point (detector/transporter.py:78-120, 217-226, 301).
 //   sub_*             longitudinal diffusion only (off by default, not in the reference): every point becomes one
 //                     record per time bucket of its window ("sub-points"), which the deposit kernel takes as points.
-//   deposit_kernel    one CTA per work unit, one lane per mesh row: pad lookup, bivariate-normal share, accumulation
-//                     per (pad, time bucket) in a shared-memory open-addressing table that is appended to the event's
-//                     entry list in dense segments (detector/transporter.py:11-41, 123-249, 252-317; pairing.py:6-28).
+//   deposit_kernel    persistent CTAs that pull work units, one lane per mesh row: pad lookup, bivariate-normal share,
+//                     accumulation per (pad, time bucket) in a shared-memory open-addressing table that is appended to
+//                     the event's entry list in dense segments (detector/transporter.py:11-41, 123-249, 252-317; pairing.py:6-28).
 //   collect/scan/emit TB wiggle, 0 <= tb < 512 mask, canonical (ascending time bucket, pad) order, CSR compaction
 //                     (detector/simulator.py:19-49, 104-115); optional Spyral rows (detector/writer.py:61-112).
 //
@@ -1429,8 +1429,11 @@ __device__ __forceinline__ unsigned long long smem_charge_of(const SmemTable& t,
     return ((unsigned long long)hi << 32) | t.lo[slot];
 }
 
-// One CTA per work unit (a slice of one event's points, all tracks together; label = last track in `indices` order
-// to touch a key, detector/transporter.py:166-169, 247-249 = the highest rank, kept with an atomicMax).
+// Persistent CTAs, as many as are resident at once: each pulls work units from `cursor` (zeroed before every launch),
+// the chunk's groups one after the other and every group's units in its longest-first unit_order.  A unit is a slice
+// of one event's points, all tracks together; label = last track in `indices` order to touch a key,
+// detector/transporter.py:166-169, 247-249 = the highest rank, kept with an atomicMax.  The table is cleared once
+// when the CTA starts; every segment append clears the slots it reads, so each unit leaves the table empty.
 //
 // A warp takes three active points per pass; lane (s, i) owns row i (one x of the 10x10 mesh) of point s and walks
 // the ten y of that row in the reference's pixel order.  Neighbouring pixels of a row usually fall on the same pad, so
@@ -1442,234 +1445,262 @@ __device__ __forceinline__ unsigned long long smem_charge_of(const SmemTable& t,
 // and at the end; events deposited in several segments (dense events, events split over several units) may then list
 // a key several times, which order_kernel merges after sorting.
 __global__ void __launch_bounds__(DEPOSIT_THREADS, 4)
-deposit_kernel(const __grid_constant__ SimParams P, PointBuf pb, GroupView chunk, Counters* ctr) {
-    const GroupView gv = sub_group(chunk, blockIdx.y);
+deposit_kernel(const __grid_constant__ SimParams P, PointBuf pb, GroupView chunk, int n_groups, unsigned* cursor,
+               Counters* ctr) {
     extern __shared__ __align__(16) unsigned s_raw[];
     __shared__ unsigned s_nkeys, s_out, s_flush, s_base;
     __shared__ unsigned s_qkey[DEPOSIT_WARPS][QUEUE_SLOTS], s_qlo[DEPOSIT_WARPS][QUEUE_SLOTS],
         s_qhi[DEPOSIT_WARPS][QUEUE_SLOTS];
-    if ((int)blockIdx.x >= pb.n_units[gv.group]) return;
-    const int64_t ubase = (int64_t)gv.group * pb.max_units;
-    const int unit = pb.unit_order[ubase + blockIdx.x];
-    const int e = pb.unit_event[ubase + unit];
-    const int u_first = pb.unit_first[ubase + unit], u_count = pb.unit_count[ubase + unit];
+    // the unit the CTA works on: group s_group of the chunk, entry s_unit of its unit_order; cursor values
+    // [s_group_first, s_group_end) are the units of group s_group (thread 0's walk over the groups)
+    __shared__ int s_group, s_unit;
+    __shared__ unsigned s_group_first, s_group_end;
     SmemTable t;
     t.word = s_raw;
     t.lo = s_raw + SMEM_SLOTS;
     t.hi2 = s_raw + 2 * SMEM_SLOTS;
-    const int slot_event = gv.first_slot + e;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    HashEntry* region = gv.tables + (int64_t)(gv.chunk_e0 + e) * gv.hash_cap;
-    const int64_t base = (int64_t)gv.group * pb.group_cap;
-    constexpr int TABLE_VEC4 = (2 * SMEM_SLOTS + SMEM_SLOTS / 2) / 4;
-    auto clear_table = [&]() {
+    {
+        constexpr int TABLE_VEC4 = (2 * SMEM_SLOTS + SMEM_SLOTS / 2) / 4;
         uint4* v = reinterpret_cast<uint4*>(s_raw);
         for (int i = threadIdx.x; i < TABLE_VEC4; i += blockDim.x) v[i] = make_uint4(0u, 0u, 0u, 0u);
-    };
-    clear_table();
+    }
     if (threadIdx.x == 0) {
         s_nkeys = 0;
         s_out = 0;
         s_flush = 0;
+        s_group = -1;
+        s_group_first = 0;
+        s_group_end = 0;
     }
-    __syncthreads();
-    unsigned n_dep = 0, n_probe = 0, n_new = 0;
     const int sub = lane / MESH_N;                                  // point of the warp's triple; 3 = idle lanes 30, 31
     const int row = lane - sub * MESH_N;                            // mesh row (x index) of this lane
     // constant mesh weights: the rows differ from lane to lane, so they are read from shared memory (row stride 11
     // doubles: the ten rows start in ten different bank pairs), not through the constant cache
     __shared__ double s_w[MESH_N][MESH_N + 1];
     for (int k = threadIdx.x; k < MESH_N * MESH_N; k += blockDim.x) s_w[k / MESH_N][k % MESH_N] = P.mesh_w[k];
-    __syncthreads();
     const double* wrow = s_w[row];
-    const bool exact_mesh = gv.exact_mesh != 0;
+    const bool exact_mesh = chunk.exact_mesh != 0;
     unsigned* qkey = s_qkey[warp];
     unsigned* qlo = s_qlo[warp];
     unsigned* qhi = s_qhi[warp];
-    unsigned q_head = 0, q_tail = 0;  // warp-uniform ring positions
     const unsigned lanes_below = lanemask_lt();
+    static_assert(SMEM_SLOTS % DEPOSIT_THREADS == 0, "segment appends give every warp whole 32-slot blocks");
+    static_assert(sizeof(HashEntry) == 16 && offsetof(HashEntry, charge) == 8, "appends store entries as uint4");
+    constexpr unsigned NO_ROOM = ~0u;  // s_base of a segment that does not fit the event's region
 
-    auto drain = [&](unsigned n) {  // whole warp: insert ring entries [q_head, q_head + n), n <= 32
-        __syncwarp();
-        if ((unsigned)lane < n) {
-            const unsigned at = (q_head + (unsigned)lane) & (QUEUE_SLOTS - 1);
-            const unsigned kw = qkey[at];
-            const unsigned long long q = ((unsigned long long)qhi[at] << 32) | qlo[at];
-            const unsigned slot = smem_find(t, kw & SMEM_KEY_MASK, kw >> 28, n_new, n_probe);
-            smem_charge(t, slot, q, &ctr->overflow_charge);
-            atomicMax(&t.word[slot], kw);  // same key bits: the highest rank wins (transporter.py:247-249)
-        }
-        __syncwarp();
-        q_head += n;
-    };
-    auto publish_new_keys = [&]() {  // whole warp, before a barrier that precedes a read of s_nkeys
-        const unsigned total = __reduce_add_sync(FULL, n_new);
-        if (lane == 0 && total) atomicAdd(&s_nkeys, total);
-        n_new = 0;
-    };
-
-    // Append the table as one dense SEGMENT to the event's entry list and clear it (all threads, after a barrier that
-    // follows every warp's publish_new_keys).  The position comes from the event's entry counter, which the units
-    // of a split event share.  A key can then sit in several segments of the list: gv.mode marks such events and
-    // order_kernel merges the copies after sorting (integer adds commute, the label is a maximum).
-    auto append_segment = [&](bool last) {
-        if (threadIdx.x == 0) {
-            s_base = atomicAdd(&gv.n_entries[slot_event], s_nkeys);
-            if (!last) {
-                gv.mode[slot_event] = 1u;
-                atomicAdd(&ctr->flushes, 1ULL);
+    while (true) {
+        if (threadIdx.x == 0) {  // pull the next unit
+            const unsigned c = atomicAdd(cursor, 1u);
+            int g = s_group;
+            unsigned first = s_group_first, end = s_group_end;
+            while (c >= end && ++g < n_groups) {
+                first = end;
+                end += (unsigned)pb.n_units[chunk.group + g];
             }
+            s_group = g;
+            s_group_first = first;
+            s_group_end = end;
+            s_unit = (int)(c - first);
         }
-        __syncthreads();
-        const unsigned seg0 = s_base;
-        if (seg0 + s_nkeys > (unsigned)gv.hash_cap) {  // the list does not fit the event's region: the host grows it
-            if (threadIdx.x == 0) ctr->overflow_hash = 1;
-        } else {
-            const uint4* words = reinterpret_cast<const uint4*>(t.word);
-            for (int i = threadIdx.x; i < SMEM_SLOTS / 4; i += blockDim.x) {
-                const uint4 w4 = words[i];
-                const unsigned w[4] = {w4.x, w4.y, w4.z, w4.w};
-                const unsigned cnt = (w4.x != 0u) + (w4.y != 0u) + (w4.z != 0u) + (w4.w != 0u);
-                if (cnt) {
-                    unsigned pos = seg0 + atomicAdd(&s_out, cnt);
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-                        if (w[k])
-                            region[pos++] = HashEntry{w[k] & SMEM_KEY_MASK, w[k] >> 28, smem_charge_of(t, 4 * i + k)};
+        __syncthreads();  // (the first one also publishes the cleared table and the staged weights)
+        if (s_group >= n_groups) break;
+        const GroupView gv = sub_group(chunk, s_group);
+        const int64_t ubase = (int64_t)gv.group * pb.max_units;
+        const int unit = pb.unit_order[ubase + s_unit];
+        const int e = pb.unit_event[ubase + unit];
+        const int u_first = pb.unit_first[ubase + unit], u_count = pb.unit_count[ubase + unit];
+        const int slot_event = gv.first_slot + e;
+        HashEntry* region = gv.tables + (int64_t)(gv.chunk_e0 + e) * gv.hash_cap;
+        const int64_t base = (int64_t)gv.group * pb.group_cap;
+        unsigned n_dep = 0, n_probe = 0, n_new = 0;
+        unsigned q_head = 0, q_tail = 0;  // warp-uniform ring positions
+
+        auto drain = [&](unsigned n) {  // whole warp: insert ring entries [q_head, q_head + n), n <= 32
+            __syncwarp();
+            if ((unsigned)lane < n) {
+                const unsigned at = (q_head + (unsigned)lane) & (QUEUE_SLOTS - 1);
+                const unsigned kw = qkey[at];
+                const unsigned long long q = ((unsigned long long)qhi[at] << 32) | qlo[at];
+                const unsigned slot = smem_find(t, kw & SMEM_KEY_MASK, kw >> 28, n_new, n_probe);
+                smem_charge(t, slot, q, &ctr->overflow_charge);
+                atomicMax(&t.word[slot], kw);  // same key bits: the highest rank wins (transporter.py:247-249)
+            }
+            __syncwarp();
+            q_head += n;
+        };
+        auto publish_new_keys = [&]() {  // whole warp, before a barrier that precedes a read of s_nkeys
+            const unsigned total = __reduce_add_sync(FULL, n_new);
+            if (lane == 0 && total) atomicAdd(&s_nkeys, total);
+            n_new = 0;
+        };
+
+        // Append the table as one dense SEGMENT to the event's entry list and clear it in the same pass (all threads,
+        // after a barrier that follows every warp's publish_new_keys).  The position comes from the event's entry
+        // counter, which the units of a split event share.  A key can then sit in several segments of the list:
+        // gv.mode marks such events and order_kernel merges the copies after sorting (integer adds commute, the label
+        // is a maximum), and it sorts every list, so the order of the entries inside a segment is free.  Every warp
+        // compacts blocks of 32 consecutive slots: one shared atomic reserves the block's keys, the lanes write them
+        // as consecutive 16 B entries and zero their slots (the 16 hi2 words of a block belong to no other block).
+        auto append_segment = [&](bool last) {
+            if (threadIdx.x == 0) {
+                const unsigned n = s_nkeys;
+                const unsigned seg0 = atomicAdd(&gv.n_entries[slot_event], n);
+                s_base = seg0 + n > (unsigned)gv.hash_cap ? NO_ROOM : seg0;
+                if (s_base == NO_ROOM) ctr->overflow_hash = 1;  // the host grows the regions and redoes the launch
+                if (!last) {
+                    gv.mode[slot_event] = 1u;
+                    atomicAdd(&ctr->flushes, 1ULL);
+                }
+                s_nkeys = 0;  // (every warp read it before the barrier that precedes this call)
+                s_out = 0;
+            }
+            __syncthreads();
+            const unsigned seg0 = s_base;
+#pragma unroll 1
+            for (int b = warp * 32; b < SMEM_SLOTS; b += DEPOSIT_THREADS) {
+                const unsigned slot = (unsigned)(b + lane);
+                const unsigned w = t.word[slot];
+                const unsigned long long q = smem_charge_of(t, slot);
+                __syncwarp();  // every lane has read its hi2 word
+                t.word[slot] = 0u;
+                t.lo[slot] = 0u;
+                if (lane < 16) t.hi2[b / 2 + lane] = 0u;
+                const unsigned m = __ballot_sync(FULL, w != 0u);
+                if (m && seg0 != NO_ROOM) {  // warp-uniform
+                    unsigned at = 0;
+                    if (lane == 0) at = atomicAdd(&s_out, (unsigned)__popc(m));
+                    at = seg0 + __shfl_sync(FULL, at, 0) + __popc(m & lanes_below);
+                    if (w)  // one 16 B store (region rows are 16 B aligned; HashEntry is only 8 B aligned)
+                        reinterpret_cast<uint4*>(region)[at] =
+                            make_uint4(w & SMEM_KEY_MASK, w >> 28, (unsigned)q, (unsigned)(q >> 32));
                 }
             }
-        }
-        if (last) return;
-        __syncthreads();
-        clear_table();
-        if (threadIdx.x == 0) {
-            s_nkeys = 0;
-            s_out = 0;
-            s_flush = 0;
-        }
-        __syncthreads();
-    };
+            if (threadIdx.x == 0) s_flush = 0;  // (every warp read it before the barrier above)
+            __syncthreads();
+        };
 
-    // The unit's slice [u_first, u_first + u_count) of the event's run, all tracks together: the label of a key is
-    // the highest rank that touched it (atomicMax on the slot word), so points need no ordering.  Warps run freely:
-    // a warp that sees the table filling up raises s_flush, every warp notices at its next pass boundary and only
-    // then do they meet at a barrier (every barrier of this kernel is followed by the same uniform decision on
-    // s_flush, whichever call site a warp arrives from).
-    const int64_t run0 = pb.start[(int64_t)slot_event * pb.ranks];
-    const int end = u_first + u_count;
-    for (int p0 = u_first; p0 < end; p0 += POINTS_PER_ITER) {
-        const int w0 = p0 + warp * POINTS_PER_WARP;
-        if (w0 < end) {  // warp-uniform
-            const int pp = w0 + sub;
-            const bool have = sub < POINTS_PER_WARP && pp < end;
-            const int64_t p = base + run0 + (have ? pp : w0);
-            const uint4* rp = reinterpret_cast<const uint4*>(pb.rec + p * REC_WORDS);
-            uint4 head = __ldg(rp);
-            if (!have) head.x = 0u;
-            const unsigned r = __ldg(pb.rec + p * REC_WORDS + 14);  // rank of the point's track
-            const int kind = (int)(head.x >> 30), tb = (int)(head.x & 0x1FFFFFFFu);
-            const bool careful_point = (head.x >> 29) & 1u;
-            const unsigned keybase = (((unsigned)tb << 15) + 1u) | (r << 28);  // + pad = slot word
-            const double qd = kind == 2 ? __hiloint2double((int)head.w, (int)head.z) : 0.0;
-            const double guard = exact_mesh ? 2.0 : (double)__uint_as_float(head.y);
-            int cur = -1;         // pad of the run being summed
-            long long acc = 0;    // its charge so far
-            int pad[MESH_N];
+        // The unit's slice [u_first, u_first + u_count) of the event's run, all tracks together: the label of a key is
+        // the highest rank that touched it (atomicMax on the slot word), so points need no ordering.  Warps run
+        // freely: a warp that sees the table filling up raises s_flush, every warp notices at its next pass boundary
+        // and only then do they meet at a barrier (every barrier inside a unit is followed by the same uniform
+        // decision on s_flush, whichever call site a warp arrives from).
+        const int64_t run0 = pb.start[(int64_t)slot_event * pb.ranks];
+        const int end = u_first + u_count;
+        for (int p0 = u_first; p0 < end; p0 += POINTS_PER_ITER) {
+            const int w0 = p0 + warp * POINTS_PER_WARP;
+            if (w0 < end) {  // warp-uniform
+                const int pp = w0 + sub;
+                const bool have = sub < POINTS_PER_WARP && pp < end;
+                const int64_t p = base + run0 + (have ? pp : w0);
+                const uint4* rp = reinterpret_cast<const uint4*>(pb.rec + p * REC_WORDS);
+                uint4 head = __ldg(rp);
+                if (!have) head.x = 0u;
+                const unsigned r = __ldg(pb.rec + p * REC_WORDS + 14);  // rank of the point's track
+                const int kind = (int)(head.x >> 30), tb = (int)(head.x & 0x1FFFFFFFu);
+                const bool careful_point = (head.x >> 29) & 1u;
+                const unsigned keybase = (((unsigned)tb << 15) + 1u) | (r << 28);  // + pad = slot word
+                const double qd = kind == 2 ? __hiloint2double((int)head.w, (int)head.z) : 0.0;
+                const double guard = exact_mesh ? 2.0 : (double)__uint_as_float(head.y);
+                int cur = -1;         // pad of the run being summed
+                long long acc = 0;    // its charge so far
+                int pad[MESH_N];
 #pragma unroll
-            for (int j = 0; j < MESH_N; ++j) pad[j] = -1;
-            if (kind != 0) {
-                // pad-table row of this lane's mesh row, columns of the ten mesh columns (make_point)
-                const uint4 cols = __ldg(rp + 1);
-                const uint2 tail = __ldg(reinterpret_cast<const uint2*>(rp + 2));  // iy[8], iy[9] | ix[0], ix[1]
-                const int ix = (int)__ldg(reinterpret_cast<const int16_t*>(rp) + 18 + row);
-                const unsigned cw[5] = {cols.x, cols.y, cols.z, cols.w, tail.x};
-                const int16_t* lut_row = P.lut + (int64_t)max(ix, 0) * P.lut_n;
-                if (kind == 2) {
+                for (int j = 0; j < MESH_N; ++j) pad[j] = -1;
+                if (kind != 0) {
+                    // pad-table row of this lane's mesh row, columns of the ten mesh columns (make_point)
+                    const uint4 cols = __ldg(rp + 1);
+                    const uint2 tail = __ldg(reinterpret_cast<const uint2*>(rp + 2));  // iy[8], iy[9] | ix[0], ix[1]
+                    const int ix = (int)__ldg(reinterpret_cast<const int16_t*>(rp) + 18 + row);
+                    const unsigned cw[5] = {cols.x, cols.y, cols.z, cols.w, tail.x};
+                    const int16_t* lut_row = P.lut + (int64_t)max(ix, 0) * P.lut_n;
+                    if (kind == 2) {
 #pragma unroll
-                    for (int j = 0; j < MESH_N; ++j) {  // all pad lookups first: independent loads in flight
-                        const int iy = (j & 1) ? (int)cw[j / 2] >> 16 : (int)(int16_t)(cw[j / 2] & 0xFFFFu);
-                        if (ix >= 0 && iy >= 0) pad[j] = (int)__ldg(lut_row + iy);
-                    }
-                } else if (row == 0) {  // detector/transporter.py:123-169: all electrons on one pad
-                    const int iy = (int)(int16_t)(cw[0] & 0xFFFFu);
-                    if (ix >= 0 && iy >= 0) cur = (int)__ldg(lut_row + iy);
-                    acc = (long long)__hiloint2double((int)head.w, (int)head.z);
-                    n_dep += cur >= 0;
-                }
-            }
-            // detector/transporter.py:240-246: int(pdf * step^2 * electrons).  pdf * step^2 is the constant mesh
-            // weight up to rounding (see make_point); the reference's own expression is evaluated only where the
-            // rounding could change the truncation -- rare, so the warp then takes a second copy of the loop.
-            unsigned risky = 0u;
-            const bool careful_warp = __any_sync(FULL, careful_point);
-            if (careful_warp && careful_point) {
-#pragma unroll
-                for (int j = 0; j < MESH_N; ++j) {
-                    const double v = __dmul_rn(wrow[j], qd);
-                    if (!(fabs(__dsub_rn(v, rint(v))) > __dmul_rn(guard, v)) && pad[j] >= 0) risky |= 1u << j;
-                }
-            }
-            const double* g = pb.geom + p * GEOM_DOUBLES;
-            auto walk_row = [&](auto careful) {
-                // j == MESH_N is the sentinel that pushes the last run of the row
-#pragma unroll
-                for (int j = 0; j <= MESH_N; ++j) {
-                    const int pj = j < MESH_N ? pad[j] : -1;
-                    long long share = 0;  // (of a pixel without pad: added to a run that is never pushed)
-                    if (j < MESH_N) {
-                        share = (long long)__dmul_rn(wrow[j], qd);
-                        if (decltype(careful)::value) {
-                            if ((risky >> j) & 1u) share = exact_share(g, row, j);
+                        for (int j = 0; j < MESH_N; ++j) {  // all pad lookups first: independent loads in flight
+                            const int iy = (j & 1) ? (int)cw[j / 2] >> 16 : (int)(int16_t)(cw[j / 2] & 0xFFFFu);
+                            if (ix >= 0 && iy >= 0) pad[j] = (int)__ldg(lut_row + iy);
                         }
-                        n_dep += pj >= 0;
+                    } else if (row == 0) {  // detector/transporter.py:123-169: all electrons on one pad
+                        const int iy = (int)(int16_t)(cw[0] & 0xFFFFu);
+                        if (ix >= 0 && iy >= 0) cur = (int)__ldg(lut_row + iy);
+                        acc = (long long)__hiloint2double((int)head.w, (int)head.z);
+                        n_dep += cur >= 0;
                     }
-                    const bool change = pj != cur;
-                    const bool push = change && cur >= 0;
-                    const unsigned m = __ballot_sync(FULL, push);
-                    if (m) {  // warp-uniform
-                        if (push) {
-                            const unsigned at = (q_tail + __popc(m & lanes_below)) & (QUEUE_SLOTS - 1);
-                            qkey[at] = keybase + (unsigned)cur;
-                            qlo[at] = (unsigned)acc;
-                            qhi[at] = (unsigned)((unsigned long long)acc >> 32);
-                        }
-                        q_tail += __popc(m);
-                        if (q_tail - q_head >= 32u) drain(32u);
-                    }
-                    if (change) {
-                        cur = pj;
-                        acc = 0;
-                    }
-                    acc += share;
                 }
-            };
-            if (careful_warp && __any_sync(FULL, risky != 0u)) walk_row(std::true_type{});
-            else walk_row(std::false_type{});
+                // detector/transporter.py:240-246: int(pdf * step^2 * electrons).  pdf * step^2 is the constant mesh
+                // weight up to rounding (see make_point); the reference's own expression is evaluated only where the
+                // rounding could change the truncation -- rare, so the warp then takes a second copy of the loop.
+                unsigned risky = 0u;
+                const bool careful_warp = __any_sync(FULL, careful_point);
+                if (careful_warp && careful_point) {
+#pragma unroll
+                    for (int j = 0; j < MESH_N; ++j) {
+                        const double v = __dmul_rn(wrow[j], qd);
+                        if (!(fabs(__dsub_rn(v, rint(v))) > __dmul_rn(guard, v)) && pad[j] >= 0) risky |= 1u << j;
+                    }
+                }
+                const double* g = pb.geom + p * GEOM_DOUBLES;
+                auto walk_row = [&](auto careful) {
+                    // j == MESH_N is the sentinel that pushes the last run of the row
+#pragma unroll
+                    for (int j = 0; j <= MESH_N; ++j) {
+                        const int pj = j < MESH_N ? pad[j] : -1;
+                        long long share = 0;  // (of a pixel without pad: added to a run that is never pushed)
+                        if (j < MESH_N) {
+                            share = (long long)__dmul_rn(wrow[j], qd);
+                            if (decltype(careful)::value) {
+                                if ((risky >> j) & 1u) share = exact_share(g, row, j);
+                            }
+                            n_dep += pj >= 0;
+                        }
+                        const bool change = pj != cur;
+                        const bool push = change && cur >= 0;
+                        const unsigned m = __ballot_sync(FULL, push);
+                        if (m) {  // warp-uniform
+                            if (push) {
+                                const unsigned at = (q_tail + __popc(m & lanes_below)) & (QUEUE_SLOTS - 1);
+                                qkey[at] = keybase + (unsigned)cur;
+                                qlo[at] = (unsigned)acc;
+                                qhi[at] = (unsigned)((unsigned long long)acc >> 32);
+                            }
+                            q_tail += __popc(m);
+                            if (q_tail - q_head >= 32u) drain(32u);
+                        }
+                        if (change) {
+                            cur = pj;
+                            acc = 0;
+                        }
+                        acc += share;
+                    }
+                };
+                if (careful_warp && __any_sync(FULL, risky != 0u)) walk_row(std::true_type{});
+                else walk_row(std::false_type{});
+            }
+            publish_new_keys();
+            if (*(volatile unsigned*)&s_nkeys > (unsigned)gv.spill_keys) *(volatile unsigned*)&s_flush = 1u;
+            if (__any_sync(FULL, *(volatile unsigned*)&s_flush != 0u)) {
+                __syncthreads();
+                append_segment(false);
+            }
         }
+        while (q_tail != q_head) drain(min(32u, q_tail - q_head));
         publish_new_keys();
         if (*(volatile unsigned*)&s_nkeys > (unsigned)gv.spill_keys) *(volatile unsigned*)&s_flush = 1u;
-        if (__any_sync(FULL, *(volatile unsigned*)&s_flush != 0u)) {
+        while (true) {
             __syncthreads();
+            if (*(volatile unsigned*)&s_flush == 0u) break;
             append_segment(false);
         }
-    }
-    while (q_tail != q_head) drain(min(32u, q_tail - q_head));
-    publish_new_keys();
-    if (*(volatile unsigned*)&s_nkeys > (unsigned)gv.spill_keys) *(volatile unsigned*)&s_flush = 1u;
-    while (true) {
-        __syncthreads();
-        if (*(volatile unsigned*)&s_flush == 0u) break;
-        append_segment(false);
-    }
-    append_segment(true);
-    unsigned long long n_dep64 = n_dep, n_probe64 = n_probe + (lane == 0 ? q_tail : 0u);  // q_tail: runs pushed = inserts
-    for (int o = 16; o > 0; o >>= 1) {
-        n_dep64 += __shfl_xor_sync(FULL, n_dep64, o);
-        n_probe64 += __shfl_xor_sync(FULL, n_probe64, o);
-    }
-    if (lane == 0 && n_dep64) {
-        atomicAdd(&ctr->deposits, n_dep64);
-        atomicAdd(&ctr->probes, n_probe64);
+        append_segment(true);  // leaves the table empty and s_nkeys, s_out, s_flush zero for the next unit
+        unsigned long long n_dep64 = n_dep, n_probe64 = n_probe + (lane == 0 ? q_tail : 0u);  // q_tail: runs pushed = inserts
+        for (int o = 16; o > 0; o >>= 1) {
+            n_dep64 += __shfl_xor_sync(FULL, n_dep64, o);
+            n_probe64 += __shfl_xor_sync(FULL, n_probe64, o);
+        }
+        if (lane == 0 && n_dep64) {
+            atomicAdd(&ctr->deposits, n_dep64);
+            atomicAdd(&ctr->probes, n_probe64);
+        }
     }
 }
 
