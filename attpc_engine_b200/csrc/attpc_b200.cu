@@ -550,6 +550,14 @@ float sum_ms(const std::vector<std::pair<cudaEvent_t, cudaEvent_t>>& marks) {
     return total;
 }
 
+// The Spyral rows of a call: float64 rows, or (`typed`, ATTPC_SPYRAL_COLUMNS) the typed columns.
+SpyralSink spyral_sink(AttpcSim* sim, bool typed) {
+    if (typed)
+        return {nullptr, nullptr, sim->rcol_pad.d(), sim->rcol_tbq.d(), sim->rcol_elo.d(), sim->rcol_ehi.d(),
+                sim->rcol_label.d()};
+    return {sim->rows.d(), sim->row_labels.d(), nullptr, nullptr, nullptr, nullptr, nullptr};
+}
+
 SpyralArgs spyral_args(AttpcSim* sim, int64_t first, int64_t n_events, bool typed, bool keep_all, const Counters* ctr) {
     SpyralArgs sa;
     memset(&sa, 0, sizeof sa);
@@ -564,18 +572,10 @@ SpyralArgs spyral_args(AttpcSim* sim, int64_t first, int64_t n_events, bool type
     sa.cloud_cap = std::min<int64_t>(sim->labels.dev.n / sim->labels.row_bytes, sa.scratch_rows);
     sa.kept = sim->row_kept.p;
     sa.row_offsets = sim->row_offsets_dev.p;
-    sa.rows = sim->rows.d();
-    sa.row_labels = sim->row_labels.d();
+    sa.sink = spyral_sink(sim, typed);
     sa.sort_keys = sim->row_sort_keys.p;
     sa.sort_idx = sim->row_sort_idx.p;
     sa.keep_all = keep_all ? 1 : 0;
-    if (typed) {
-        sa.out_pad = sim->rcol_pad.d();
-        sa.out_tb_q16 = sim->rcol_tbq.d();
-        sa.out_e_lo = sim->rcol_elo.d();
-        sa.out_e_hi = sim->rcol_ehi.d();
-        sa.out_label = sim->rcol_label.d();
-    }
     return sa;
 }
 
@@ -754,19 +754,10 @@ FinalizeArgs finalize_args(AttpcSim* sim, const LaunchPlan& plan, const OutputPl
         }
     }
     if (op.spy_fused) {
-        fa.spyral = op.spy_cols ? 1u : 2u;
+        fa.spyral = true;
         fa.row_kept = sim->row_kept.p + b0;
         fa.row_offsets = sim->row_offsets_dev.p + b0;
-        if (op.spy_cols) {
-            fa.rcol_pad = sim->rcol_pad.d();
-            fa.rcol_tb_q16 = sim->rcol_tbq.d();
-            fa.rcol_e_lo = sim->rcol_elo.d();
-            fa.rcol_e_hi = sim->rcol_ehi.d();
-            fa.rcol_label = sim->rcol_label.d();
-        } else {
-            fa.rows = sim->rows.d();
-            fa.row_labels = sim->row_labels.d();
-        }
+        fa.rsink = spyral_sink(sim, op.spy_cols);
     }
     fa.replay = plan.uniforms;
     if (fa.replay.offsets) fa.replay.offsets += b0;

@@ -150,6 +150,46 @@ struct HashEntry {
     unsigned long long charge;
 };
 
+// ------------------------------------------------------------------------------------------------ block scans
+// Exclusive scan of one value per thread of a CTA of T threads; returns the thread's prefix, `total` for everybody.
+// Every thread calls it, and the last read of s_warp [T / 32] must be behind a barrier; one barrier.
+template <int T, typename V>
+__device__ __forceinline__ V block_scan(V v, V& total, V* s_warp) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    V incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const V t = __shfl_up_sync(FULL, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    V base = incl - v;
+    total = 0;
+#pragma unroll
+    for (int w = 0; w < T / 32; ++w) {
+        const V t = s_warp[w];
+        if (w < warp) base += t;
+        total += t;
+    }
+    return base;
+}
+
+// Exclusive scan of load(0), ..., load(n - 1) on top of `base` in tiles of T values: store(i, base + sum of the values
+// before i).  Every thread of the CTA calls it and gets the final sum.  Value i is loaded and stored by one thread.
+template <int T, typename V, typename Load, typename Store>
+__device__ __forceinline__ V scan_tiles(int n, V base, V* s_warp, Load load, Store store) {
+    for (int start = 0; start < n; start += T) {
+        const int i = start + (int)threadIdx.x;
+        V total;
+        __syncthreads();  // (the previous tile is done with s_warp)
+        const V before = block_scan<T>(i < n ? load(i) : V(0), total, s_warp);
+        if (i < n) store(i, base + before);
+        base += total;
+    }
+    return base;
+}
+
 // ----------------------------------------------------------------------------------------------- stopping power
 struct TableView {
     const double* t;
@@ -435,27 +475,9 @@ track_plan_count_kernel(const __grid_constant__ SimParams P, const __grid_consta
 
 // (2) exclusive scan of the counts, class-major (one CTA)
 __global__ void __launch_bounds__(1024) track_plan_scan_kernel(unsigned* cta_counts, int n) {
-    __shared__ unsigned s_part[1024];
-    __shared__ unsigned s_base;
-    const int tid = threadIdx.x;
-    if (tid == 0) s_base = 0;
-    __syncthreads();
-    for (int start = 0; start < n; start += 1024) {
-        const int i = start + tid;
-        const unsigned v = i < n ? cta_counts[i] : 0u;
-        s_part[tid] = v;
-        __syncthreads();
-        for (int o = 1; o < 1024; o <<= 1) {
-            const unsigned add = tid >= o ? s_part[tid - o] : 0u;
-            __syncthreads();
-            s_part[tid] += add;
-            __syncthreads();
-        }
-        if (i < n) cta_counts[i] = s_base + s_part[tid] - v;
-        __syncthreads();
-        if (tid == 0) s_base += s_part[1023];
-        __syncthreads();
-    }
+    __shared__ unsigned s_warp[32];
+    scan_tiles<1024>(n, 0u, s_warp, [&](int i) { return cta_counts[i]; },
+                     [&](int i, unsigned s) { cta_counts[i] = s; });
 }
 
 // (3) stable scatter: position = start of (class, CTA) + tracks of the same class before this one in the CTA
@@ -999,8 +1021,7 @@ constexpr int GEOM_DOUBLES = 12;
 // size so that the longest start first (the per-event cost varies by 100x between a short recoil and a stopped ion).
 __global__ void __launch_bounds__(1024) point_scan_kernel(PointBuf pb, GroupView chunk, const Counters* ctr) {
     const GroupView gv = sub_group(chunk, blockIdx.x);
-    __shared__ unsigned s_part[1024];
-    __shared__ unsigned s_base, s_ubase;
+    __shared__ unsigned s_warp[32];
     __shared__ uint32_t s_sort[MAX_UNITS_SORT];
     const int tid = threadIdx.x;
     if (ctr->overflow_points) {  // the point lists are incomplete: the host will redo the launch with bigger buffers
@@ -1013,46 +1034,21 @@ __global__ void __launch_bounds__(1024) point_scan_kernel(PointBuf pb, GroupView
     int32_t* u_first = pb.unit_first + (int64_t)gv.group * pb.max_units;
     int32_t* u_count = pb.unit_count + (int64_t)gv.group * pb.max_units;
     int32_t* u_order = pb.unit_order + (int64_t)gv.group * pb.max_units;
-    if (tid == 0) {
-        s_base = 0;
-        s_ubase = 0;
-    }
-    __syncthreads();
-    for (int start = 0; start < n; start += 1024) {
-        const int i = start + tid;
-        const unsigned v = i < n ? pb.cnt[first + i] : 0u;
-        s_part[tid] = v;
-        __syncthreads();
-        for (int o = 1; o < 1024; o <<= 1) {
-            const unsigned add = tid >= o ? s_part[tid - o] : 0u;
-            __syncthreads();
-            s_part[tid] += add;
-            __syncthreads();
-        }
-        if (i < n) pb.start[first + i] = s_base + s_part[tid] - v;
-        __syncthreads();
-        if (tid == 0) s_base += s_part[1023];
-        __syncthreads();
-    }
+    scan_tiles<1024>(n, 0u, s_warp, [&](int i) { return pb.cnt[first + i]; },
+                     [&](int i, unsigned s) { pb.start[first + i] = s; });
     // units: event e has ceil(points / UNIT_POINTS) of them (at least one, so that empty events still get their
     // zero-length entry list written)
-    for (int start = 0; start < gv.n_events; start += 1024) {
-        const int e = start + tid;
-        unsigned pts = 0;
-        if (e < gv.n_events)
+    const unsigned up = (unsigned)pb.unit_points;
+    unsigned pts = 0, nu = 0;  // of the thread's event: scan_tiles loads and stores it on the same thread
+    const unsigned n_units = scan_tiles<1024>(
+        gv.n_events, 0u, s_warp,
+        [&](int e) {
+            pts = 0;
             for (int r = 0; r < pb.ranks; ++r) pts += pb.cnt[first + (int64_t)e * pb.ranks + r];
-        const unsigned up = (unsigned)pb.unit_points;
-        const unsigned nu = e < gv.n_events ? max(1u, (pts + up - 1u) / up) : 0u;
-        s_part[tid] = nu;
-        __syncthreads();
-        for (int o = 1; o < 1024; o <<= 1) {
-            const unsigned add = tid >= o ? s_part[tid - o] : 0u;
-            __syncthreads();
-            s_part[tid] += add;
-            __syncthreads();
-        }
-        if (e < gv.n_events) {
-            unsigned u0 = s_ubase + s_part[tid] - nu;
+            nu = max(1u, (pts + up - 1u) / up);
+            return nu;
+        },
+        [&](int e, unsigned u0) {
             gv.mode[gv.first_slot + e] = nu > 1 ? 1u : 0u;  // several units: a key may be listed once per unit
             for (unsigned k = 0; k < nu; ++k) {
                 const unsigned u = u0 + k;
@@ -1062,12 +1058,9 @@ __global__ void __launch_bounds__(1024) point_scan_kernel(PointBuf pb, GroupView
                     u_count[u] = (int32_t)min(up, pts - min(pts, k * up));
                 }
             }
-        }
-        __syncthreads();
-        if (tid == 0) s_ubase += s_part[1023];
-        __syncthreads();
-    }
-    const int total = min((int)s_ubase, pb.max_units);
+        });
+    __syncthreads();  // (the sort reads the unit counts of every thread)
+    const int total = min((int)n_units, pb.max_units);
     if (tid == 0) pb.n_units[gv.group] = total;
     // longest first: bitonic sort of (UNIT_POINTS - count) << 16 | unit ... only when it fits the sort buffer
     if (total <= MAX_UNITS_SORT) {
@@ -1201,6 +1194,27 @@ __device__ __noinline__ long long exact_share(const double* g, int i, int j) {
     return (long long)__dmul_rn(__dmul_rn(pdf, cell2), g[10]);
 }
 
+// The record of a point of track rank `rank` (make_point's arguments) at ordered position d of `pb`, with its mesh
+// constants when the record is careful.
+__device__ __forceinline__ void put_point(const SimParams& P, const PointBuf& pb, int64_t d, double cx, double cy,
+                                          double time, int tb, long long q, int rank, bool exact_mesh) {
+    double g[GEOM_DOUBLES];
+    uint32_t rec[REC_WORDS];
+#pragma unroll
+    for (int k = 0; k < GEOM_DOUBLES; ++k) g[k] = 0.0;
+    make_point(P, cx, cy, time, tb, q, exact_mesh, g, rec);
+    rec[14] = (uint32_t)rank;
+    if ((rec[0] >> 29) & 1u) {  // only the exact path of the deposit kernel reads the mesh constants
+        double2* out = reinterpret_cast<double2*>(pb.geom + d * GEOM_DOUBLES);
+#pragma unroll
+        for (int k = 0; k < GEOM_DOUBLES / 2; ++k) out[k] = make_double2(g[2 * k], g[2 * k + 1]);
+    }
+    uint4* out_rec = reinterpret_cast<uint4*>(pb.rec + d * REC_WORDS);
+#pragma unroll
+    for (int k = 0; k < REC_WORDS / 4; ++k)
+        out_rec[k] = make_uint4(rec[4 * k], rec[4 * k + 1], rec[4 * k + 2], rec[4 * k + 3]);
+}
+
 // Scatter the group's points into (event, rank, arrival) order and compute their mesh constants (one thread each).
 __global__ void __launch_bounds__(256) point_order_kernel(const __grid_constant__ SimParams P, PointBuf pb,
                                                           GroupView chunk, const Counters* ctr) {
@@ -1211,20 +1225,7 @@ __global__ void __launch_bounds__(256) point_order_kernel(const __grid_constant_
     for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (int64_t)gridDim.x * blockDim.x) {
         const int64_t i = base + p;
         const int64_t d = base + pb.start[(int64_t)pb.ev[i] * pb.ranks + pb.rank[i]] + pb.j[i];
-        double g[GEOM_DOUBLES];
-        uint32_t rec[REC_WORDS];
-#pragma unroll
-        for (int k = 0; k < GEOM_DOUBLES; ++k) g[k] = 0.0;
-        make_point(P, pb.x[i], pb.y[i], pb.t[i], (int)pb.t[i], pb.q[i], gv.exact_mesh != 0, g, rec);
-        rec[14] = (uint32_t)pb.rank[i];
-        if ((rec[0] >> 29) & 1u) {  // only the exact path of the deposit kernel reads the mesh constants
-            double2* out = reinterpret_cast<double2*>(pb.geom + d * GEOM_DOUBLES);
-#pragma unroll
-            for (int k = 0; k < GEOM_DOUBLES / 2; ++k) out[k] = make_double2(g[2 * k], g[2 * k + 1]);
-        }
-        uint4* out_rec = reinterpret_cast<uint4*>(pb.rec + d * REC_WORDS);
-#pragma unroll
-        for (int k = 0; k < REC_WORDS / 4; ++k) out_rec[k] = make_uint4(rec[4 * k], rec[4 * k + 1], rec[4 * k + 2], rec[4 * k + 3]);
+        put_point(P, pb, d, pb.x[i], pb.y[i], pb.t[i], (int)pb.t[i], pb.q[i], pb.rank[i], gv.exact_mesh != 0);
     }
 }
 
@@ -1336,23 +1337,9 @@ __global__ void __launch_bounds__(256) sub_point_kernel(const __grid_constant__ 
         int k0, k1;
         long_window(P, time, sl, k0, k1);
         int64_t d = sbase + sb.start[l] + nsub[base + pb.start[l] + pb.j[i]];
-        for (int k = k0; k <= k1; ++k, ++d) {
-            double g[GEOM_DOUBLES];
-            uint32_t rec[REC_WORDS];
-#pragma unroll
-            for (int m = 0; m < GEOM_DOUBLES; ++m) g[m] = 0.0;
-            make_point(P, cx, cy, time, k, sl > 0.0 ? long_electrons(time, sl, k, q) : q, gv.exact_mesh != 0, g, rec);
-            rec[14] = (uint32_t)pb.rank[i];
-            if ((rec[0] >> 29) & 1u) {
-                double2* out = reinterpret_cast<double2*>(sb.geom + d * GEOM_DOUBLES);
-#pragma unroll
-                for (int m = 0; m < GEOM_DOUBLES / 2; ++m) out[m] = make_double2(g[2 * m], g[2 * m + 1]);
-            }
-            uint4* out_rec = reinterpret_cast<uint4*>(sb.rec + d * REC_WORDS);
-#pragma unroll
-            for (int m = 0; m < REC_WORDS / 4; ++m)
-                out_rec[m] = make_uint4(rec[4 * m], rec[4 * m + 1], rec[4 * m + 2], rec[4 * m + 3]);
-        }
+        for (int k = k0; k <= k1; ++k, ++d)
+            put_point(P, sb, d, cx, cy, time, k, sl > 0.0 ? long_electrons(time, sl, k, q) : q, pb.rank[i],
+                      gv.exact_mesh != 0);
     }
 }
 
@@ -1711,6 +1698,21 @@ struct ReplayUniforms {
     const double* vals;
 };
 
+// Where Spyral rows go: the eight float64 columns of detector/writer.py:97-110 and the labels, or
+// (ATTPC_SPYRAL_COLUMNS: pad != null) what those are functions of: pad, time bucket Q16.16, electrons as 32 low +
+// 16 high bits, label.
+// Amplitude and integral follow from the electrons alone, x / y / pad size from the pad id and z from the time bucket,
+// so the host rebuilds the eight columns bit for bit (Engine.rows_from_columns).
+struct SpyralSink {
+    double* rows;  // [rows, 8]
+    int64_t* row_labels;
+    int16_t* pad;
+    uint32_t* tb_q16;
+    uint32_t* e_lo;
+    uint16_t* e_hi;
+    int8_t* label;
+};
+
 struct FinalizeArgs {
     uint64_t seed;
     int64_t first_event;      // global id of event slot 0 of the launch batch
@@ -1757,22 +1759,38 @@ struct FinalizeArgs {
         unsigned* count;
         unsigned* cursor;
     } big, far;  // big: second shared-memory tier; far: lists ordered in global scratch
-    // Spyral rows of the same events (detector/writer.py:61-112, 232-238), thresholded and in z order: 0 = none,
-    // 1 = typed columns (rcol_*), 2 = float64 rows
-    uint32_t spyral, pad_;
+    // Spyral rows of the same events (detector/writer.py:61-112, 232-238), thresholded and in z order, into rsink
+    bool spyral;
     unsigned* row_kept;       // [launch events] rows above the ADC threshold
     int64_t* row_offsets;     // [launch events + 1]
-    double* rows;             // [out_cap, 8]
-    int64_t* row_labels;
-    int16_t* rcol_pad;
-    uint32_t* rcol_tb_q16;
-    uint32_t* rcol_e_lo;
-    uint16_t* rcol_e_hi;
-    int8_t* rcol_label;
+    SpyralSink rsink;         // [out_cap] rows
 };
 
 constexpr uint32_t F_KEEP_ALL_TB = 1u, F_SPYRAL = 2u, F_NO_WIGGLE = 4u;
 constexpr int TB_BINS = 1024;  // counting-sort bins over the integer time bucket (last bin collects tb >= 1023)
+
+// Exclusive scan, in place, of a[at(0)], a[at(1)], ..., a[at(TB_BINS - 1)]; every thread of the CTA calls it after a
+// barrier that completed `a`; returns the total; ends with a barrier.
+template <int T, typename Map>
+__device__ __forceinline__ unsigned scan_bins(unsigned* a, Map at, unsigned* s_warp) {
+    constexpr int PER = TB_BINS / T;
+    const int tid = threadIdx.x;
+    unsigned local[PER], sum = 0;
+#pragma unroll
+    for (int k = 0; k < PER; ++k) {
+        local[k] = a[at(tid * PER + k)];
+        sum += local[k];
+    }
+    unsigned total;
+    unsigned base = block_scan<T>(sum, total, s_warp);
+#pragma unroll
+    for (int k = 0; k < PER; ++k) {
+        a[at(tid * PER + k)] = base;
+        base += local[k];
+    }
+    __syncthreads();
+    return total;
+}
 
 __device__ __forceinline__ double wiggle_of(const FinalizeArgs& fa, int slot_event, unsigned key, Counters* ctr) {
     if (fa.flags & F_NO_WIGGLE) return 0.0;
@@ -1801,18 +1819,9 @@ struct SpyralArgs {
     int64_t scratch_rows;     // rows of sort_keys / sort_idx per half
     const Counters* ctr;      // launch counters (null: none): a launch that overflowed a buffer is void and will be redone
     int64_t cloud_cap;        // rows the cloud buffer holds
-    // typed sink (ATTPC_SPYRAL_COLUMNS): pad, time bucket Q16.16, electrons as 32 low + 16 high bits, label; null = the
-    // float64 rows below.  Amplitude and integral follow from the electrons alone, x / y / pad size from the pad id and
-    // z from the time bucket, so the host rebuilds the eight columns bit for bit (engine.SimBatch.spyral_rows).
-    int16_t* out_pad;
-    uint32_t* out_tb_q16;
-    uint32_t* out_e_lo;
-    uint16_t* out_e_hi;
-    int8_t* out_label;
     unsigned* kept;           // [n_events]
     int64_t* row_offsets;     // [n_events + 1]
-    double* rows;             // [n, 8] (capacity = input points)
-    int64_t* row_labels;
+    SpyralSink sink;          // [n] rows (capacity = input points)
     uint64_t* sort_keys;      // [n] scratch (order-preserving bits of z)
     uint32_t* sort_idx;       // [n] scratch
     int32_t keep_all;         // 1: every row, input order (plain convert_to_spyral, detector/writer.py:61-112)
@@ -1832,6 +1841,41 @@ __device__ __forceinline__ void shaped(const SimParams& P, double electrons, dou
     // (explicitly rounded operations: the host rebuilds this value from the typed columns and must get the same bits)
     integral = __dadd_rn(__dmul_rn(4095.0, (double)lo),
                          __dmul_rn(electrons, __dsub_rn(P.resp_prefix[P.n_response], P.resp_prefix[lo])));
+}
+
+// detector/writer.py:101-103: (window_edge - tb) / (window_edge - mm_edge) * length * 1000.0 (explicitly rounded, like
+// the amplitude: the host rebuilds it from the typed columns)
+__device__ __forceinline__ double spyral_z(const SimParams& P, double tbf) {
+    const double span = (double)(P.win_edge - P.mm_edge);
+    return __dmul_rn(__dmul_rn(__ddiv_rn(__dsub_rn(P.win_edge, tbf), span), P.length), 1000.0);
+}
+
+// Spyral row `at` of `sink` (detector/writer.py:97-110) from a cloud row: `pad` and `electrons` as the float64 cloud
+// holds them, `tbf` the time bucket with its wiggle and `tb_q16` that value in Q16.16.
+__device__ __forceinline__ void put_spyral_row(const SimParams& P, const SpyralSink& sink, int64_t at, double pad,
+                                               double tbf, uint32_t tb_q16, double electrons, int64_t label) {
+    const int p = (int)pad;
+    if (sink.pad) {
+        const unsigned long long q = (unsigned long long)(long long)electrons;
+        sink.pad[at] = (int16_t)p;
+        sink.tb_q16[at] = tb_q16;
+        sink.e_lo[at] = (uint32_t)q;
+        sink.e_hi[at] = (uint16_t)(q >> 32);
+        sink.label[at] = (int8_t)label;
+        return;
+    }
+    double amp, integral;
+    shaped(P, electrons, amp, integral);
+    double* row = sink.rows + at * 8;
+    row[0] = P.pad_xy[2 * p];
+    row[1] = P.pad_xy[2 * p + 1];
+    row[2] = spyral_z(P, tbf);
+    row[3] = amp;
+    row[4] = integral;
+    row[5] = pad;
+    row[6] = tbf;
+    row[7] = P.pad_scale[p];
+    sink.row_labels[at] = label;
 }
 
 __device__ __forceinline__ uint64_t orderable(double v) {
@@ -1862,32 +1906,15 @@ __global__ void __launch_bounds__(256) spyral_count_kernel(const __grid_constant
 }
 
 __global__ void __launch_bounds__(1024) spyral_scan_kernel(SpyralArgs sa) {
-    __shared__ unsigned long long s_part[1024];
-    __shared__ unsigned long long s_base;
-    const int tid = threadIdx.x;
-    if (tid == 0) s_base = *sa.total;
-    __syncthreads();
-    sa.kept += sa.first;
-    sa.row_offsets += sa.first;
-    for (int64_t start = 0; start < sa.n_events; start += 1024) {
-        const int64_t i = start + tid;
-        const unsigned long long v = i < sa.n_events ? sa.kept[i] : 0ULL;
-        s_part[tid] = v;
-        __syncthreads();
-        for (int o = 1; o < 1024; o <<= 1) {
-            const unsigned long long add = tid >= o ? s_part[tid - o] : 0ULL;
-            __syncthreads();
-            s_part[tid] += add;
-            __syncthreads();
-        }
-        if (i < sa.n_events) sa.row_offsets[i] = (int64_t)(s_base + s_part[tid] - v);
-        __syncthreads();
-        if (tid == 0) s_base += s_part[1023];
-        __syncthreads();
-    }
-    if (tid == 0) {
-        sa.row_offsets[sa.n_events] = (int64_t)s_base;
-        *sa.total = s_base;
+    __shared__ unsigned long long s_warp[32];
+    const unsigned* kept = sa.kept + sa.first;
+    int64_t* row_offsets = sa.row_offsets + sa.first;
+    const unsigned long long total =
+        scan_tiles<1024>((int)sa.n_events, *sa.total, s_warp, [&](int i) { return (unsigned long long)kept[i]; },
+                         [&](int i, unsigned long long s) { row_offsets[i] = (int64_t)s; });
+    if (threadIdx.x == 0) {
+        row_offsets[sa.n_events] = (int64_t)total;
+        *sa.total = total;
     }
 }
 
@@ -1910,7 +1937,6 @@ spyral_rows_kernel(const __grid_constant__ SimParams P, SpyralArgs sa) {
     const int64_t out0 = sa.row_offsets[e];
     const int n = (int)sa.kept[e];
     if (n == 0) return;
-    const double span = (double)(P.win_edge - P.mm_edge);
     const int64_t total = sa.scratch_rows;
     uint64_t* stash_k = sa.sort_keys + a;           // unordered survivors
     uint32_t* stash_v = sa.sort_idx + a;
@@ -1925,43 +1951,18 @@ spyral_rows_kernel(const __grid_constant__ SimParams P, SpyralArgs sa) {
             const double amp = fmin(__dmul_rn(P.resp_max, sa.cloud[i * 3 + 2]), 4095.0);
             if (amp > P.adc_threshold) {
                 const double tbf = sa.cloud[i * 3 + 1];
-                // detector/writer.py:101-103: (window_edge - tb) / (window_edge - mm_edge) * length * 1000.0
-                const double z = __dmul_rn(__dmul_rn(__ddiv_rn(__dsub_rn(P.win_edge, tbf), span), P.length), 1000.0);
                 const unsigned pos = atomicAdd(&s_n, 1u);
-                stash_k[pos] = orderable(z);
+                stash_k[pos] = orderable(spyral_z(P, tbf));
                 stash_v[pos] = (uint32_t)(i - a);
                 const int tbi = min(max((int)tbf, 0), TB_BINS - 1);
                 atomicAdd(&s_hist[TB_BINS - 1 - tbi], 1u);
             }
         }
         __syncthreads();
-        {
-            const int b0 = threadIdx.x * (TB_BINS / 256);
-            unsigned local[TB_BINS / 256], sum = 0;
-#pragma unroll
-            for (int k = 0; k < TB_BINS / 256; ++k) {
-                local[k] = s_hist[b0 + k];
-                sum += local[k];
-            }
-            unsigned incl = sum;
-            const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-            for (int o = 1; o < 32; o <<= 1) {
-                const unsigned v = __shfl_up_sync(FULL, incl, o);
-                if (lane >= o) incl += v;
-            }
-            if (lane == 31) s_warp[warp] = incl;
-            __syncthreads();
-            unsigned base = incl - sum;
-            for (int w = 0; w < warp; ++w) base += s_warp[w];
-#pragma unroll
-            for (int k = 0; k < TB_BINS / 256; ++k) {
-                s_hist[b0 + k] = base;
-                s_fill[b0 + k] = base;
-                base += local[k];
-            }
-            if (threadIdx.x == 255) s_hist[TB_BINS] = base;
-            __syncthreads();
-        }
+        const unsigned kept = scan_bins<256>(s_hist, [](int b) { return b; }, s_warp);
+        for (int i = threadIdx.x; i < TB_BINS; i += blockDim.x) s_fill[i] = s_hist[i];
+        if (threadIdx.x == 0) s_hist[TB_BINS] = kept;
+        __syncthreads();
         for (int i = threadIdx.x; i < n; i += blockDim.x) {
             const uint32_t id = stash_v[i];
             const int tbi = min(max((int)sa.cloud[(a + id) * 3 + 1], 0), TB_BINS - 1);
@@ -1987,29 +1988,8 @@ spyral_rows_kernel(const __grid_constant__ SimParams P, SpyralArgs sa) {
             for (int j = lo; j < hi; ++j) before += keys[j] < kv || (keys[j] == kv && idx[j] < id);
             place = lo + before;
         }
-        const int pad = (int)padf;
-        if (sa.out_pad) {  // typed columns: what the eight columns are functions of
-            const int64_t at = out0 + place;
-            const unsigned long long q = (unsigned long long)(long long)el;
-            sa.out_pad[at] = (int16_t)pad;
-            sa.out_tb_q16[at] = (uint32_t)(tbf * 65536.0);  // exact for the library's 16-bit wiggle
-            sa.out_e_lo[at] = (uint32_t)q;
-            sa.out_e_hi[at] = (uint16_t)(q >> 32);
-            sa.out_label[at] = (int8_t)sa.labels[src];
-            continue;
-        }
-        double amp, integral;
-        shaped(P, el, amp, integral);
-        double* row = sa.rows + (out0 + place) * 8;
-        row[0] = P.pad_xy[2 * pad];
-        row[1] = P.pad_xy[2 * pad + 1];
-        row[2] = __dmul_rn(__dmul_rn(__ddiv_rn(__dsub_rn(P.win_edge, tbf), span), P.length), 1000.0);
-        row[3] = amp;
-        row[4] = integral;
-        row[5] = padf;
-        row[6] = tbf;
-        row[7] = P.pad_scale[pad];
-        sa.row_labels[out0 + place] = sa.labels[src];
+        // (tb_q16 is exact for the library's 16-bit wiggle)
+        put_spyral_row(P, sa.sink, out0 + place, padf, tbf, (uint32_t)(tbf * 65536.0), el, sa.labels[src]);
     }
 }
 
@@ -2051,66 +2031,6 @@ struct FinShared {
     unsigned warp[32];
     unsigned keys, next;
 };
-
-// Exclusive scan, in place, of a[at(0)], a[at(1)], ..., a[at(TB_BINS - 1)]; every thread of the CTA calls it after a
-// barrier that completed `a`; returns the total; ends with a barrier.
-template <int T, typename Map>
-__device__ __forceinline__ unsigned scan_bins(unsigned* a, Map at, unsigned* s_warp) {
-    constexpr int PER = TB_BINS / T;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    unsigned local[PER], sum = 0;
-#pragma unroll
-    for (int k = 0; k < PER; ++k) {
-        local[k] = a[at(tid * PER + k)];
-        sum += local[k];
-    }
-    unsigned incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const unsigned v = __shfl_up_sync(FULL, incl, o);
-        if (lane >= o) incl += v;
-    }
-    if (lane == 31) s_warp[warp] = incl;
-    __syncthreads();
-    unsigned base = incl - sum, total = 0;
-#pragma unroll
-    for (int w = 0; w < T / 32; ++w) {
-        const unsigned v = s_warp[w];
-        if (w < warp) base += v;
-        total += v;
-    }
-#pragma unroll
-    for (int k = 0; k < PER; ++k) {
-        a[at(tid * PER + k)] = base;
-        base += local[k];
-    }
-    __syncthreads();
-    return total;
-}
-
-// Exclusive scan of one value per thread; returns the thread's prefix, `total` for everybody; two barriers.
-template <int T>
-__device__ __forceinline__ unsigned scan_threads(unsigned v, unsigned& total, unsigned* s_warp) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    unsigned incl = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const unsigned t = __shfl_up_sync(FULL, incl, o);
-        if (lane >= o) incl += t;
-    }
-    __syncthreads();  // (the previous use of s_warp is over)
-    if (lane == 31) s_warp[warp] = incl;
-    __syncthreads();
-    unsigned base = incl - v;
-    total = 0;
-#pragma unroll
-    for (int w = 0; w < T / 32; ++w) {
-        const unsigned t = s_warp[w];
-        if (w < warp) base += t;
-        total += t;
-    }
-    return base;
-}
 
 template <typename Item, bool SMEM, int T>
 __device__ __forceinline__ void order_event(const SimParams& P, const FinalizeArgs& fa, const GroupView& chunk,
@@ -2205,16 +2125,8 @@ __device__ __forceinline__ void order_event(const SimParams& P, const FinalizeAr
             if (lane == 0) H[p >> 5] = m;
         }
         __syncthreads();
-        const int n_words = (n + 31) >> 5;
-        unsigned done = 0;
-        for (int w0 = 0; w0 < n_words; w0 += T) {
-            const int w = w0 + tid;
-            unsigned total;
-            const unsigned before = scan_threads<T>(w < n_words ? (unsigned)__popc(H[w]) : 0u, total, sh.warp);
-            if (w < n_words) HP[w] = done + before;
-            done += total;
-        }
-        n_rows = (int)done;
+        n_rows = (int)scan_tiles<T>((n + 31) >> 5, 0u, sh.warp, [&](int w) { return (unsigned)__popc(H[w]); },
+                                    [&](int w, unsigned s) { HP[w] = s; });
         __syncthreads();
     }
     auto is_row = [&](int p) -> bool { return !dup || ((H[p >> 5] >> (p & 31)) & 1u); };
@@ -2223,7 +2135,7 @@ __device__ __forceinline__ void order_event(const SimParams& P, const FinalizeAr
     // sinks once the offsets of all events are known).  Charge and label of a row fold the copies of its key:
     // integer adds commute, the label is the highest rank (detector/transporter.py:166-169, 247-249).
     uint4* staged = fa.staged + (int64_t)L * chunk.hash_cap;
-    const bool spy = fa.spyral != 0u;
+    const bool spy = fa.spyral;
     const bool draw = fa.replay.offsets == nullptr;  // (replayed uniforms have 53 bits: emit_kernel looks them up)
     for (int p = tid; p < n; p += T) {
         Item w_out = 0;
@@ -2345,41 +2257,22 @@ order_queue_kernel(const __grid_constant__ SimParams P, const __grid_constant__ 
 // top of the totals of the call so far.  One CTA: a thread sums a run of consecutive events, the CTA scans the sums.
 __global__ void __launch_bounds__(1024) offsets_kernel(FinalizeArgs fa, GroupView chunk, Counters* ctr) {
     __shared__ unsigned long long s_warp[2][32];
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
     const int n = chunk.n_events;
     const int per = (n + 1023) / 1024;
     const int e0 = min(n, tid * per), e1 = min(n, e0 + per);
-    const bool spy = fa.spyral != 0u;
+    const bool spy = fa.spyral;
     const unsigned* kept = fa.kept + chunk.first_slot;
     const unsigned* rkept = fa.row_kept + chunk.first_slot;
-    unsigned long long sum[2] = {0ULL, 0ULL};
+    unsigned long long sum[2] = {0ULL, 0ULL}, base[2], total[2];
     for (int e = e0; e < e1; ++e) {
         sum[0] += kept[e];
         if (spy) sum[1] += rkept[e];
     }
-    unsigned long long incl[2] = {sum[0], sum[1]};
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1)
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-            const unsigned long long v = __shfl_up_sync(FULL, incl[c], o);
-            if (lane >= o) incl[c] += v;
-        }
-    if (lane == 31) {
-        s_warp[0][warp] = incl[0];
-        s_warp[1][warp] = incl[1];
-    }
-    __syncthreads();
-    unsigned long long base[2], total[2];
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
-        base[c] = fa.csr_total[2 * c] + incl[c] - sum[c];
-        total[c] = fa.csr_total[2 * c];
-        for (int w = 0; w < 32; ++w) {
-            const unsigned long long v = s_warp[c][w];
-            if (w < warp) base[c] += v;
-            total[c] += v;
-        }
+        base[c] = fa.csr_total[2 * c] + block_scan<1024>(sum[c], total[c], s_warp[c]);
+        total[c] += fa.csr_total[2 * c];
     }
     __syncthreads();  // (every thread has read csr_total)
     int64_t* offsets = fa.offsets + chunk.first_slot;
@@ -2416,11 +2309,10 @@ emit_kernel(const __grid_constant__ SimParams P, const __grid_constant__ Finaliz
     const int n = (int)fa.kept[slot_event];
     const int64_t off = fa.offsets[slot_event];
     if (off + n > fa.out_cap) return;  // (offsets_kernel has raised overflow_out)
-    const bool spy = fa.spyral != 0u && fa.row_offsets[slot_event] + (int64_t)fa.row_kept[slot_event] <= fa.out_cap;
+    const bool spy = fa.spyral && fa.row_offsets[slot_event] + (int64_t)fa.row_kept[slot_event] <= fa.out_cap;
     const int64_t roff = fa.spyral ? fa.row_offsets[slot_event] : 0;
     const uint4* staged = fa.staged + (int64_t)L * chunk.hash_cap;
     const bool replayed = fa.replay.offsets != nullptr;
-    const double span = (double)(P.win_edge - P.mm_edge);
     const bool packed = fa.col_wiggle != nullptr;
     __shared__ unsigned s_tb[NUM_TB];  // packed columns: rows of the event per time bucket
     if (packed) {
@@ -2478,29 +2370,9 @@ emit_kernel(const __grid_constant__ SimParams P, const __grid_constant__ Finaliz
                 }
             }
         }
-        if (spy && (s.z >> 31)) {
-            const int64_t at = roff + (s.w >> 4);
-            if (fa.rcol_pad) {  // typed columns: what the eight columns are functions of
-                fa.rcol_pad[at] = (int16_t)pad;
-                fa.rcol_tb_q16[at] = (tb << 16) | u16;
-                fa.rcol_e_lo[at] = (uint32_t)q;
-                fa.rcol_e_hi[at] = (uint16_t)(q >> 32);
-                fa.rcol_label[at] = (int8_t)label;
-            } else {
-                double amp, integral;
-                shaped(P, (double)(long long)q, amp, integral);
-                double* row = fa.rows + at * 8;
-                row[0] = P.pad_xy[2 * pad];
-                row[1] = P.pad_xy[2 * pad + 1];
-                row[2] = __dmul_rn(__dmul_rn(__ddiv_rn(__dsub_rn(P.win_edge, tbf), span), P.length), 1000.0);
-                row[3] = amp;
-                row[4] = integral;
-                row[5] = (double)pad;
-                row[6] = tbf;
-                row[7] = P.pad_scale[pad];
-                fa.row_labels[at] = label;
-            }
-        }
+        if (spy && (s.z >> 31))
+            put_spyral_row(P, fa.rsink, roff + (s.w >> 4), (double)pad, tbf, (tb << 16) | u16, (double)(long long)q,
+                           label);
     }
     if (packed) {
         __syncthreads();

@@ -409,6 +409,17 @@ def test_spyral_columns_rebuild_the_float64_rows(name, n):
                              copy_events_per_launch=16)  # fmt: skip
     assert np.array_equal(chunked.row_offsets, full.row_offsets) and np.array_equal(chunked.rows, full.rows)
     assert np.array_equal(chunked.cloud, full.cloud)
+    # unmasked time buckets: the Spyral pass over the float64 cloud writes the typed columns instead of finalize
+    from attpc_engine_b200.detector.engine import engine_for
+    from attpc_engine_b200.detector.simulator import _nuclei_for
+
+    eng = engine_for(cfg, _nuclei_for(zs, as_, idx, nuclear_map))
+    wide = eng.simulate_batch(m, v, zs, as_, idx, seed=17, spyral_rows=True, keep_all_tb=True)
+    wide_cols = eng.simulate_batch(m, v, zs, as_, idx, seed=17, spyral_rows=True, keep_all_tb=True, row_columns=True,
+                                   rows_only=True)  # fmt: skip
+    assert wide_cols.row_columns is not None and wide_cols.stats["n_rows"] == wide.stats["n_rows"] > 0
+    assert np.array_equal(wide_cols.row_offsets, wide.row_offsets)
+    assert np.array_equal(wide_cols.rows, wide.rows) and np.array_equal(wide_cols.row_labels, wide.row_labels)
 
 
 @pytest.mark.parametrize("compact", [True, False])
