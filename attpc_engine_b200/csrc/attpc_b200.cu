@@ -1359,6 +1359,12 @@ int attpc_create(const AttpcConfig* cfg, const int16_t* pad_lut, const double* p
         g_create_error = "attpc_create: windows_edge == micromegas_edge, drift_velocity <= 0 or w_value <= 0";
         return ATTPC_E_BADARG;
     }
+    // a point drifts for up to windows_edge time buckets, and the 28-bit table key holds 13 bits of time bucket: a
+    // wider window would lose the points beyond bucket 8191 without a word (ATTPC_KEEP_ALL_TB keeps them otherwise)
+    if (cfg->windows_edge > 8191) {
+        g_create_error = "attpc_create: windows_edge must be <= 8191 (time buckets are kept in 13 bits)";
+        return ATTPC_E_BADARG;
+    }
     if (!(cfg->longitudinal_diffusion >= 0.0) || !std::isfinite(cfg->longitudinal_diffusion)) {
         g_create_error = "attpc_create: longitudinal_diffusion must be finite and >= 0";
         return ATTPC_E_BADARG;

@@ -591,10 +591,12 @@ class Engine:
         keep_all_tb: bool = False,
         no_wiggle: bool = False,
         spyral_rows: bool = False,
+        host_copy: bool = True,
     ) -> tuple[SimBatch, list[np.ndarray]]:
         """Everything after the trajectory from given rows and random numbers (parity part (a)).
 
         ``uniforms[e] = (keys, u)`` replays `simulator.py:108` keyed by Szudzik id.
+        ``host_copy=False``: the rows stay on the device, as in `simulate_batch` (`read_device_result` fetches them).
         Returns the batch and, per track, ``electrons`` as `solver.py:343-346` would.
         """
         n_tracks = len(tracks)
@@ -629,6 +631,7 @@ class Engine:
             (_lib.KEEP_ALL_TB if keep_all_tb else 0)
             | (_lib.NO_WIGGLE if no_wiggle else 0)
             | (_lib.SPYRAL_ROWS if spyral_rows else 0)
+            | (0 if host_copy else _lib.SKIP_HOST_COPY)
             | self._mesh_flag()
         )
         res = _lib.AttpcResult()
@@ -639,7 +642,7 @@ class Engine:
         )  # fmt: skip
         _lib.check(code, self.handle)
         del keep
-        batch = self._collect(res, 0, True, spyral_rows)
+        batch = self._collect(res, 0, True, spyral_rows and host_copy)
         per_track = [electrons[offsets[t] : offsets[t + 1]].copy() for t in range(n_tracks)]
         return batch, per_track
 

@@ -71,7 +71,7 @@ typedef struct AttpcConfig {
     double w_value;         /* eV */
     double gas_density;     /* g/cm^3, GasTarget.density */
     int32_t micromegas_edge;
-    int32_t windows_edge;
+    int32_t windows_edge;   /* <= 8191: attpc_create returns ATTPC_E_BADARG otherwise */
     double adc_threshold;
     double drift_velocity;  /* m / time bucket, Config.drift_velocity */
     double grid_low_mm;     /* pad_grid_edges[0] */
